@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this build (libipdm_b200.so), one rank per GPU
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host CPU (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's result, to compare two builds
 
 A "step" is one pass of the whole hot path over one batch of synthetic slices per GPU:
 projection-domain guided process (t_start_proj) -> FBP -> sharpen -> image-domain guided process
@@ -50,7 +51,26 @@ def parse():
     ap.add_argument("--skip_cpu_whole_slice", action="store_true", help="do not run the one unsampled whole slice on the host (~150 s)")
     ap.add_argument("--skip_extras", action="store_true", help="only the headline line: no modes / c1 / cuda_graph / C4 / C5 sub-reports")
     ap.add_argument("--cuda_graph", type=int, default=0, help="1: capture the whole progressive pass in one CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's denoised images, float32) as DIR/denoised_images.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, images):
+    """Saves the [B,1,512,512] result of the last timed step; beyond DUMP_LIMIT_BYTES only the leading slices are kept."""
+    import numpy as np
+    per_slice = images[0].numel() * 4
+    images = images[:max(1, DUMP_LIMIT_BYTES // per_slice)]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "denoised_images.npy"), images.float().cpu().numpy())
 
 
 def peaks():
@@ -308,6 +328,8 @@ def run_b200(args, rank, world, local_rank):
     if args.cuda_graph and launches == 0 and args.warmup > 0:
         launches = launches_first_step * args.steps                  # replays do not pass through the host-side launch counter
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)           # before any later call can reuse the result's memory
     step_e2e()
     ms_e2e, _ = timed(step_e2e, args.steps)
     if world > 1:

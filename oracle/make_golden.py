@@ -12,7 +12,9 @@ Every case fixes (weights seed, input seed, noise-tape seed); tests re-create th
 inputs from the same seeds (ipdm-pytorch_b200/synthetic.py) and compare the CUDA
 path and the oracle restatement against the arrays stored here.
 """
+import glob
 import importlib.util
+import io
 import json
 import os
 import sys
@@ -303,11 +305,36 @@ def TTsharpen(x, n):
     return TT.tensor_sharpen(x, n)
 
 
+FILE_LIMIT = 1_000_000           # bytes per stored file: a full-size case is split over several files
+
+
+def _npz_bytes(key, value):
+    buf = io.BytesIO()
+    np.savez_compressed(buf, **{key: value})
+    return buf.getbuffer().nbytes
+
+
 def save(name, d):
+    """Writes the arrays of one case as <name>.npz, <name>.1.npz, ... (first fit, each file under FILE_LIMIT); the tests'
+    golden(name) merges them.  Every array is stored whole."""
     os.makedirs(GOLD, exist_ok=True)
-    path = os.path.join(GOLD, name + ".npz")
-    np.savez_compressed(path, **d)
-    print(f"wrote {path} ({os.path.getsize(path) / 1024:.0f} KiB)", flush=True)
+    for stale in glob.glob(os.path.join(GOLD, glob.escape(name) + ".[0-9]*.npz")):
+        os.remove(stale)
+    parts, sizes = [], []
+    for key, value in d.items():
+        n = _npz_bytes(key, value)
+        assert n < FILE_LIMIT, (name, key, n)
+        i = next((i for i, s in enumerate(sizes) if s + n < FILE_LIMIT), len(parts))
+        if i == len(parts):
+            parts.append({})
+            sizes.append(0)
+        parts[i][key] = value
+        sizes[i] += n
+    for i, part in enumerate(parts):
+        path = os.path.join(GOLD, name + (f".{i}" if i else "") + ".npz")
+        np.savez_compressed(path, **part)
+        assert os.path.getsize(path) < FILE_LIMIT, path
+        print(f"wrote {path} ({os.path.getsize(path) / 1024:.0f} KiB)", flush=True)
 
 
 def main():

@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -17,7 +18,15 @@ def pytest_configure(config):
 
 
 def golden(name):
-    return np.load(os.path.join(GOLDEN, name + ".npz"))
+    """Arrays of tests/golden/<name>.npz merged with those of its parts <name>.1.npz, <name>.2.npz, ... (oracle/make_golden.py
+    splits a case over several files to keep each file under 1 MB)."""
+    paths = [os.path.join(GOLDEN, name + ".npz")] + sorted(glob.glob(os.path.join(GOLDEN, glob.escape(name) + ".[0-9]*.npz")))
+    arrays = {}
+    for path in paths:
+        with np.load(path) as z:
+            assert not set(z.files) & set(arrays), path
+            arrays.update((k, z[k]) for k in z.files)
+    return arrays
 
 
 def rel_l2(a, b):
