@@ -89,6 +89,12 @@ int ipdm_fbp_forward(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev,
 int ipdm_fbp_convert_host(ipdm_fbp_plan* plan, const float* sino_host, float* img_host, int batch, int flip);
 /* host copies of the tables, for parity tests: theta[2000] f64, nda[912], h_RL[1823], wcos[912] */
 int ipdm_fbp_tables(const ipdm_fbp_plan* plan, double* theta, float* nda, float* h_rl, float* wcos);
+/* Forward projector in the plan's geometry (no counterpart in the reference; its projector is the Windows-only
+ * TASART2DNSL0.pyd): mu image img [B,512,512] (1/cm) -> line integrals sino [B,2000,912], the rays the backprojector reads
+ * (fan angle nda[k] + da/2), Joseph's method (one linearly interpolated sample per column or row crossed, fp32).
+ * flip as for ipdm_fbp_forward: 1 = image in the convertor's output frame, sinogram in its input frame; 0 = both native.
+ * Uses the plan's workspace (grown on demand). */
+int ipdm_fbp_project(ipdm_fbp_plan* plan, const float* img_dev, float* sino_dev, int batch, int flip, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Diffusion schedule.  Replaces Model/model.py: cosine_beta_schedule :366-372 and
@@ -144,6 +150,13 @@ int ipdm_set_noise_epoch(uint64_t epoch, void* stream);
 /* out = a*x + b*N(0,1) with caller noise or Philox (q_sample) */
 int ipdm_q_sample(const float* x_dev, const float* noise_dev, float* out_dev, float a, float b, size_t n_per_slice,
                   int batch, uint64_t seed, uint64_t call_id, void* stream);
+/* Dose-reduction noise of the reference's Utils/Low_dose_CT_simulate.py add_noise (:38-44) on line integrals p:
+ *   out = p + sqrt((1-f) e^p (1 + (1+f) Ne e^p / (f N0)) / (f N0)) * n,  f = dose in (0, 1], Ne = 5.8, N0 = 1.4e5,
+ * clamped at 0 iff clip.  n from noise_dev (same layout as sino) or, when noise_dev == NULL, from Philox4x32-10 keyed by
+ * (seed, slice id, element / 4); slice_ids_dev_or_null [B] holds the slice ids (NULL: 0..B-1), so a slice's noise does not depend
+ * on its position in the batch.  The device-resident noise epoch is not part of the key.  out_dev may alias sino_dev. */
+int ipdm_low_dose_noise(const float* sino_dev, const float* noise_dev, float* out_dev, int batch, size_t n_per_slice, float dose,
+                        int clip, uint64_t seed, const uint64_t* slice_ids_dev_or_null, void* stream);
 /* Lambda-exponent map of the first proj iteration: relu(avgpool_ks(|x-img| - median)) -> exp(amp*.) -> curve.
  * curve_kind 0 = proj_curv_init, 1 = curve_init.  out [B][H/ks][W/ks].  median_out_dev (optional) [B]. */
 int ipdm_delta_lambda_map(const float* x_dev, const float* img_dev, float* lam_exp_out_dev, float* median_out_dev,

@@ -4,6 +4,11 @@
 [B,2000,912] / [2000,912] in, the same kind out, [B,512,512] float32 ON THE HOST.  The arithmetic
 (cosine weighting, ramp filter, pixel-driven fan-beam backprojection) runs in libipdm_b200.so;
 `convert_device` is the additive zero-copy entry the progressive pipeline uses.
+
+Additive: `project(img, flip=True)` / `project_device(img)`, the forward projector in the same geometry
+(Joseph's method, see include/ipdm_b200.h ipdm_fbp_project).  It is not the reference's `proj_torch`
+(an area-integral projector with a lookup table, Recon/TASART2DNSL0.py), so the two do not agree sample
+for sample.
 """
 import numpy as np
 import torch
@@ -28,6 +33,20 @@ class FBP:
         """[B,2000,912] CUDA tensor -> [B,512,512] CUDA tensor, no host copy, current stream."""
         with torch.cuda.device(self.device):
             return self._plan.forward(pj.contiguous().float(), flip=flip)
+
+    def project_device(self, img, flip=True):
+        """[B,512,512] CUDA mu image -> [B,2000,912] CUDA line integrals, no host copy, current stream."""
+        with torch.cuda.device(self.device):
+            return self._plan.project(img.contiguous().float(), flip=flip)
+
+    def project(self, img, flip=True):
+        """`convert`'s contract in the other direction: ndarray or Tensor [B,512,512] / [512,512] in, the same kind out,
+        [B,2000,912] float32 on the host."""
+        as_tensor = isinstance(img, torch.Tensor)
+        x = img.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(img, dtype=np.float32))
+        x = x[None] if x.dim() == 2 else x
+        out = self.project_device(x.to(self.device), flip).cpu()
+        return out if as_tensor else out.numpy()
 
     def convert(self, pj, flip=True):
         as_tensor = isinstance(pj, torch.Tensor)

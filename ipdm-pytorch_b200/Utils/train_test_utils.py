@@ -7,6 +7,8 @@ attributes (`ResultTempDict`s of numpy arrays keyed `iter_k`), so `main.py` and 
 drive it unchanged.  Differences, all additive:
   * batches of B >= 1 slices are accepted everywhere; statistics are per slice (SURVEY D3);
   * `progressive_denoiser(..., noise=(proj_tape, img_tape))` injects caller noise for parity runs;
+  * `simulate_low_dose` makes low-dose inputs from full-dose images or sinograms on the device, and the
+    option of the same name makes `test()` use it instead of reading low-dose files;
   * between the projection stage, the FBP convertor, the sharpen filter and the image stage the
     data stays on the GPU (the reference crosses to the host three times, SURVEY 3.2);
   * training (`train`, the train branch of `fit`), figures and skimage/piq metrics are out of scope.
@@ -154,7 +156,7 @@ class progressive_domain_denoiser:
 
     # ---- in-kernel noise keys ----------------------------------------------------------------
     def _stage_seed(self, stage):
-        """Philox key of one stage (0 proj, 1 img, 2 ultra): a hash of (noise_seed, stage), so that neighbouring seeds (e.g. the
+        """Philox key of one stage (0 proj, 1 img, 2 ultra, 3 low-dose simulation): a hash of (noise_seed, stage), so that neighbouring seeds (e.g. the
         per-rank seeds of bench.py) never share a stream with another stage."""
         z = (int(getattr(self.opt, "noise_seed", 0)) * 0x9E3779B97F4A7C15 + (stage + 1) * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
         z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
@@ -255,17 +257,42 @@ class progressive_domain_denoiser:
         self.noise_strength = ns
         return res
 
-    def _convert_device(self, sino):
-        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan."""
+    def _reserve_fbp(self, batch):
         if self._fbp is None:
             self.convertor(None)
-        G = 10 if self.opt.clip_proj else 1
-        if sino.shape[0] > getattr(self, "_fbp_cap", 0):            # the plan re-allocates its filtered-sinogram workspace for a larger batch
+        if batch > getattr(self, "_fbp_cap", 0):                     # the plan re-allocates its filtered-sinogram workspace for a larger batch
             if not torch.cuda.is_current_stream_capturing():
                 self._drop_graph()
-            self._fbp_cap = int(sino.shape[0])
+            self._fbp_cap = int(batch)
+
+    def _convert_device(self, sino):
+        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan."""
+        self._reserve_fbp(sino.shape[0])
+        G = 10 if self.opt.clip_proj else 1
         s = sino[:, 0].float()
         return self._fbp.convert_device(s * G if G != 1 else s)[:, None]
+
+    def simulate_low_dose(self, fd, dose=None, slice_ids=None):
+        """Low-dose inputs at `dose` (default opt.dose) from a full-dose batch: a sinogram [B,1,2000,912] gets the dose-reduction
+        noise of the reference's Low_dose_CT_simulate.add_noise; a mu image [B,1,512,512] is forward-projected (FBP geometry,
+        Joseph's method) first.  Returns (ldproj [B,1,2000,912], ldct [B,1,512,512] = FBP of ldproj, no sharpen), both on the
+        device.  The noise is drawn in line-integral units from Philox keyed by (a hash of noise_seed, slice id, bin), slice ids
+        default to 0..B-1; with clip_proj, sinograms are in the dataset's units (line integrals / 10) on the way in and out."""
+        o = self.opt
+        fd = fd.to(o.device).float()
+        if fd.dim() != 4 or fd.shape[1] != 1:
+            raise ValueError(f"simulate_low_dose: expected [B,1,2000,912] or [B,1,512,512], got {tuple(fd.shape)}")
+        G = 10 if o.clip_proj else 1
+        self._reserve_fbp(fd.shape[0])
+        if tuple(fd.shape[2:]) == (_eng.N_PIX, _eng.N_PIX):
+            sino = self._fbp.project_device(fd[:, 0])
+        elif tuple(fd.shape[2:]) == (_eng.N_VIEWS, _eng.N_DET):
+            sino = fd[:, 0] * G                                                # always a fresh buffer: the noise is added in place
+        else:
+            raise ValueError(f"simulate_low_dose: expected [B,1,2000,912] or [B,1,512,512], got {tuple(fd.shape)}")
+        _eng.low_dose_noise(sino, o.dose if dose is None else dose, seed=self._stage_seed(3), slice_ids=slice_ids, clip=True, out=sino)
+        ldproj = (sino / G if G != 1 else sino)[:, None]
+        return ldproj, self._convert_device(ldproj)
 
     def _img_stage(self, x, noise=None, noise_strength=None):
         o = self.opt
@@ -511,6 +538,11 @@ class progressive_domain_denoiser:
 
     def _run_batch(self, epoch, ids, cols):
         ld_img, fd_proj, fd_img, ld_proj = cols
+        if getattr(self.opt, "simulate_low_dose", False):                    # LD files on disk, if any, are not used
+            fd = fd_proj if fd_proj is not None else fd_img
+            if fd is None:
+                raise ValueError("simulate_low_dose needs full-dose projections or images in the test dataset")
+            ld_proj, ld_img = self.simulate_low_dose(fd, slice_ids=[int(i) for i in ids])
         self.temp_clear()
         self.data_sample_load(ldct=ld_img, ldproj=ld_proj, fdproj=fd_proj, fdct=fd_img)
         if self.opt.mode == "test_proj":

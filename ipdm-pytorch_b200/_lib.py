@@ -50,6 +50,9 @@ _SIGNATURES = {
     "ipdm_fbp_forward": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
     "ipdm_fbp_convert_host": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int]),
     "ipdm_fbp_tables": (ctypes.c_int, [vp, vp, vp, vp, vp]),
+    "ipdm_fbp_project": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
+    "ipdm_low_dose_noise": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_size_t, ctypes.c_float, ctypes.c_int, ctypes.c_uint64, vp,
+                                           vp]),
     "ipdm_cosine_beta_schedule": (ctypes.c_int, [ctypes.c_int, ctypes.c_double, c_double_p]),
     "ipdm_schedule_at": (ctypes.c_int, [ctypes.c_int, ctypes.c_double, ctypes.c_int, c_double_p]),
     "ipdm_lincomb": (ctypes.c_int, [vp, ctypes.c_float, vp, ctypes.c_float, vp, ctypes.c_float, vp, ctypes.c_size_t, vp]),

@@ -19,7 +19,7 @@
 //           (|s/c| <= 0.6 inside the image), s/c is a Newton-refined reciprocal.  Bound: FP32 issue
 //           (about 33 instructions per pixel-view update, 524.3 M updates / slice), not HBM
 //           (8.345 MB compulsory bytes / slice; SURVEY.md D5).
-#include "common.cuh"
+#include "fbp_plan.cuh"
 
 #include <cmath>
 #include <vector>
@@ -29,29 +29,6 @@ namespace ipdm {
 constexpr int NV = IPDM_N_VIEWS, ND = IPDM_N_DET, NP = IPDM_N_PIX;
 constexpr int NHALF = ND / 2;          // 456 samples per detector parity
 constexpr int NTAP = 2 * NHALF - 1;    // 911 taps per parity class (d = -455..455)
-
-struct FbpTables {
-    std::vector<double> theta;   // [2000]
-    std::vector<float> nda;      // [912]
-    std::vector<float> h;        // [1823]
-    std::vector<float> wcos;     // [912]
-    double dtheta, D, da;
-};
-
-}  // namespace ipdm
-
-struct ipdm_fbp_plan {
-    ipdm::FbpTables host;
-    float* d_wcos = nullptr;     // [912]
-    float* d_htap = nullptr;     // [2][911]  H_c[d + 455] = h[2d + 2c - 1 + 911]
-    float2* d_cs = nullptr;      // [2000] (cos theta, sin theta) from fp64
-    float* d_work = nullptr;     // filtered sinograms [cap][2000][912]
-    int cap = 0;
-    float h0 = 0.f, inv_da = 0.f, u_off = 0.f, dtheta_f = 0.f;
-    double dtheta = 0.0;
-};
-
-namespace ipdm {
 
 // ------------------------------------------------------------------------------------------------
 // tables: same expressions as FBP.__init__ (FBP_kernel.py:32-56), evaluated in fp64 on the host
@@ -262,7 +239,7 @@ fbp_backproject_kernel(const float* __restrict__ q, float* __restrict__ img, con
     for (int p = 0; p < PX; ++p) ob[(size_t)(i_base + 8 * p) * NP + jo] = acc[p];
 }
 
-static int ensure_workspace(ipdm_fbp_plan* plan, int batch) {
+int ensure_workspace(ipdm_fbp_plan* plan, int batch) {
     if (batch <= plan->cap) return IPDM_OK;
     if (plan->d_work) IPDM_CHECK_CUDA(cudaFree(plan->d_work));
     plan->d_work = nullptr;
@@ -286,6 +263,11 @@ extern "C" int ipdm_fbp_plan_create(ipdm_fbp_plan** out, int max_batch) {
         for (int d = -455; d <= 455; ++d) htap[c * NTAP + d + 455] = t.h[2 * d + 2 * c - 1 + (ND - 1)];
     std::vector<float2> cs(NV);
     for (int v = 0; v < NV; ++v) cs[v] = make_float2((float)std::cos(t.theta[v]), (float)std::sin(t.theta[v]));
+    std::vector<float2> ray(ND);
+    for (int k = 0; k < ND; ++k) {
+        const double a = (double)t.nda[k] + 0.5 * t.da;
+        ray[k] = make_float2((float)std::cos(a), (float)std::sin(a));
+    }
     p->h0 = t.h[ND - 1];
     p->inv_da = (float)(1.0 / t.da);
     p->u_off = (float)(0.5 - (double)t.nda[0] / t.da);
@@ -293,9 +275,11 @@ extern "C" int ipdm_fbp_plan_create(ipdm_fbp_plan** out, int max_batch) {
     IPDM_CHECK_CUDA(cudaMalloc(&p->d_wcos, ND * sizeof(float)));
     IPDM_CHECK_CUDA(cudaMalloc(&p->d_htap, 2 * NTAP * sizeof(float)));
     IPDM_CHECK_CUDA(cudaMalloc(&p->d_cs, NV * sizeof(float2)));
+    IPDM_CHECK_CUDA(cudaMalloc(&p->d_ray, ND * sizeof(float2)));
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_wcos, t.wcos.data(), ND * sizeof(float), cudaMemcpyHostToDevice));
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_htap, htap.data(), 2 * NTAP * sizeof(float), cudaMemcpyHostToDevice));
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_cs, cs.data(), NV * sizeof(float2), cudaMemcpyHostToDevice));
+    IPDM_CHECK_CUDA(cudaMemcpy(p->d_ray, ray.data(), ND * sizeof(float2), cudaMemcpyHostToDevice));
     if (max_batch > 0) IPDM_CHECK(ensure_workspace(p, max_batch));
     *out = p;
     return IPDM_OK;
@@ -303,7 +287,7 @@ extern "C" int ipdm_fbp_plan_create(ipdm_fbp_plan** out, int max_batch) {
 
 extern "C" int ipdm_fbp_plan_destroy(ipdm_fbp_plan* p) {
     if (!p) return IPDM_OK;
-    cudaFree(p->d_wcos); cudaFree(p->d_htap); cudaFree(p->d_cs); cudaFree(p->d_work);
+    cudaFree(p->d_wcos); cudaFree(p->d_htap); cudaFree(p->d_cs); cudaFree(p->d_ray); cudaFree(p->d_work);
     delete p;
     return IPDM_OK;
 }

@@ -18,30 +18,16 @@
 namespace ipdm {
 
 // ------------------------------------------------------------------------------------------------
-// Philox4x32-10 + Box-Muller: 4 normals per (seed, call, slice, quad index)
+// Philox4x32-10 + Box-Muller (common.cuh): 4 normals per (seed, call, slice, quad index)
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox_round(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3, uint32_t k0, uint32_t k1) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
-}
 // Device-resident part of the Philox key.  Kernel arguments are frozen when a CUDA graph is captured, so the per-run
 // entropy lives here: ipdm_set_noise_epoch() updates it between replays (ordinary stream-ordered memcpy).
 __device__ unsigned long long d_noise_epoch = 0ull;
 
 __device__ __forceinline__ float4 philox_normal4(uint64_t seed, uint64_t call, uint32_t slice, uint32_t quad) {
-    uint32_t c0 = quad, c1 = slice, c2 = (uint32_t)call, c3 = (uint32_t)(call >> 32);
     const unsigned long long ep = d_noise_epoch;
-    uint32_t k0 = (uint32_t)seed ^ (uint32_t)(ep * 0x9E3779B97F4A7C15ull >> 32), k1 = (uint32_t)(seed >> 32) ^ (uint32_t)ep;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) { philox_round(c0, c1, c2, c3, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
-    const float s = 2.3283064365386963e-10f;                  // 2^-32
-    const float u0 = fmaf((float)c0, s, 0.5f * s), u1 = (float)c1 * s, u2 = fmaf((float)c2, s, 0.5f * s), u3 = (float)c3 * s;
-    const float r0 = sqrtf(-2.0f * __logf(u0)), r1 = sqrtf(-2.0f * __logf(u2));
-    float s0, co0, s1, co1;
-    __sincosf(6.283185307179586f * u1, &s0, &co0);
-    __sincosf(6.283185307179586f * u3, &s1, &co1);
-    return make_float4(r0 * co0, r0 * s0, r1 * co1, r1 * s1);
+    return philox_normal4_keyed(quad, slice, (uint32_t)call, (uint32_t)(call >> 32),
+                                (uint32_t)seed ^ (uint32_t)(ep * 0x9E3779B97F4A7C15ull >> 32), (uint32_t)(seed >> 32) ^ (uint32_t)ep);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -122,6 +122,18 @@ class FBPPlan:
                                                pj.shape[0], int(bool(flip))), "ipdm_fbp_convert_host")
         return out
 
+    def project(self, img, flip=True, out=None):
+        """Forward projection (Joseph's method, the geometry of `forward`): mu image [B,512,512] device (1/cm) -> line integrals
+        [B,2000,912] device.  flip as for `forward`, so forward(project(x, flip), flip) approximates x."""
+        if img.dim() != 3 or tuple(img.shape[1:]) != (N_PIX, N_PIX):
+            raise ValueError(f"image must be [B,{N_PIX},{N_PIX}], got {tuple(img.shape)}")
+        b = img.shape[0]
+        out = torch.empty(b, N_VIEWS, N_DET, device=img.device, dtype=torch.float32) if out is None else out
+        if tuple(out.shape) != (b, N_VIEWS, N_DET):
+            raise ValueError(f"out must be [{b},{N_VIEWS},{N_DET}], got {tuple(out.shape)}")
+        check(_lib.lib().ipdm_fbp_project(self._h, _dev(img, "img"), _dev(out, "out"), b, int(bool(flip)), _stream()), "ipdm_fbp_project")
+        return out
+
     def tables(self):
         theta = np.empty(N_VIEWS, np.float64)
         nda, h, wcos = np.empty(N_DET, np.float32), np.empty(2 * N_DET - 1, np.float32), np.empty(N_DET, np.float32)
@@ -194,6 +206,32 @@ def q_sample(x, a, b, noise=None, seed=0, call_id=0, out=None):
     out = torch.empty_like(x) if out is None else out
     check(_lib.lib().ipdm_q_sample(_dev(x), _opt(noise), _dev(out), float(a), float(b), x.numel() // bsz, bsz, int(seed), int(call_id),
                                    _stream()), "ipdm_q_sample")
+    return out
+
+
+def low_dose_noise(sino, dose, seed=0, slice_ids=None, noise=None, clip=True, out=None):
+    """Dose-reduction noise of the reference's add_noise (Utils/Low_dose_CT_simulate.py:38-44) on line integrals sino [B,...]
+    (device): p + sqrt((1-f) e^p (1 + (1+f) Ne e^p / (f N0)) / (f N0)) * n with f = dose, clamped at 0 iff clip.  n is the tape
+    `noise` (shaped like sino) or in-kernel Philox keyed by (seed, slice id, element / 4); slice_ids (B ints, default 0..B-1) are
+    dataset indices, so a slice draws the same noise whatever batch it is in.  out may be sino (in place)."""
+    if sino.dim() < 2:
+        raise ValueError(f"sino must be [B,...], got {tuple(sino.shape)}")
+    if not 0.0 < float(dose) <= 1.0:
+        raise ValueError(f"dose must be in (0, 1], got {dose}")
+    b = sino.shape[0]
+    out = torch.empty_like(sino) if out is None else out
+    if out.shape != sino.shape:
+        raise ValueError(f"out must be shaped like sino {tuple(sino.shape)}, got {tuple(out.shape)}")
+    if noise is not None and noise.shape != sino.shape:
+        raise ValueError(f"noise must be shaped like sino {tuple(sino.shape)}, got {tuple(noise.shape)}")
+    ids = None
+    if slice_ids is not None:
+        ids = torch.as_tensor([int(i) for i in slice_ids], dtype=torch.int64).to(sino.device)
+        if ids.numel() != b or bool((ids < 0).any()):
+            raise ValueError(f"slice_ids must hold {b} non-negative ids, got {list(slice_ids)}")
+    check(_lib.lib().ipdm_low_dose_noise(_dev(sino, "sino"), _opt(noise, "noise"), _dev(out, "out"), b, sino.numel() // b, float(dose),
+                                         int(bool(clip)), int(seed) & (2 ** 64 - 1), None if ids is None else ctypes.c_void_p(ids.data_ptr()),
+                                         _stream()), "ipdm_low_dose_noise")
     return out
 
 
