@@ -95,6 +95,19 @@ int ipdm_fbp_tables(const ipdm_fbp_plan* plan, double* theta, float* nda, float*
  * flip as for ipdm_fbp_forward: 1 = image in the convertor's output frame, sinogram in its input frame; 0 = both native.
  * Uses the plan's workspace (grown on demand). */
 int ipdm_fbp_project(ipdm_fbp_plan* plan, const float* img_dev, float* sino_dev, int batch, int flip, void* stream);
+/* Exact adjoint (transpose) of ipdm_fbp_project: sino [B,2000,912] -> img [B,512,512], img = A^T sino with A the fp32 matrix the
+ * projector applies (the same weights, bit for bit) and the same flip frames.  Deterministic (no atomics), slice by slice. */
+int ipdm_fbp_project_adjoint(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, void* stream);
+/* Ordered-subset SART convertor (replaces the SART core of the reference's Windows-only ART convertor TASART2DNSL0.pyd,
+ * correction_kernel / update_kernel; not its NSL0-TV step): line integrals sino [B,2000,912] -> mu image img [B,512,512], frames
+ * as for ipdm_fbp_forward.  Subset s = views v with v mod S = s, S = subsets dividing 2000; a sweep visits s_n = n p mod S,
+ * p the integer in [1, S) coprime to S closest to 0.382 S (smaller on a tie; 1 when S <= 2).  x0 = 0; per subset
+ * r = (b - A_s x) / R (0 where R = A 1 is 0), x <- max(0, x + relaxation * A_s^T r / C_s) where C_s = A_s^T 1 > 0.
+ * iterations >= 1 sweeps, 0 < relaxation < 2, img must not alias sino.  R and C_s are built in the plan by the first call
+ * for a given S (that call synchronises the stream and cannot be captured); later calls of the same or a smaller shape allocate
+ * nothing and do not synchronise. */
+int ipdm_fbp_sart(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets,
+                  float relaxation, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Diffusion schedule.  Replaces Model/model.py: cosine_beta_schedule :366-372 and

@@ -5,9 +5,10 @@ The flags are declared from one table instead of ~70 add_argument calls.  Refere
 purpose: `type=bool` flags are truthy for any non-empty string; a JSON overlay never overrides a
 flag that was given on the command line; `cfg_load` only merges keys that already exist and prints
 the reference's "no key names ..." line otherwise.  Additive keys of this build: `precision`
-("tf32" | "fp32" | "bf16"), `noise_seed`, `cuda_graph` and `simulate_low_dose` (the test loop makes
-its low-dose inputs from the full-dose data at `dose` instead of reading them); their defaults
-reproduce the reference.
+("tf32" | "fp32" | "bf16"), `noise_seed`, `cuda_graph`, `simulate_low_dose` (the test loop makes
+its low-dose inputs from the full-dose data at `dose` instead of reading them) and the settings of
+the `convertor="SART"` convertor, `sart_iterations` (sweeps), `sart_subsets` (S, divides 2000) and
+`sart_relaxation` (lambda in (0, 2)); their defaults reproduce the reference.
 """
 import argparse
 import json
@@ -50,7 +51,8 @@ _FLAGS = [
     ("patch_per_image", int, 4, None), ("dose", float, 0.25, None),
     # additive (B200 build)
     ("precision", str, "tf32", None), ("noise_seed", int, 0, None), ("cuda_graph", bool, False, None),
-    ("simulate_low_dose", bool, False, None),
+    ("simulate_low_dose", bool, False, None), ("sart_iterations", int, 5, None), ("sart_subsets", int, 100, None),
+    ("sart_relaxation", float, 1.0, None),
 ]
 
 

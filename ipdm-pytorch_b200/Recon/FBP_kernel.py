@@ -9,6 +9,10 @@ Additive: `project(img, flip=True)` / `project_device(img)`, the forward project
 (Joseph's method, see include/ipdm_b200.h ipdm_fbp_project).  It is not the reference's `proj_torch`
 (an area-integral projector with a lookup table, Recon/TASART2DNSL0.py), so the two do not agree sample
 for sample.
+
+Additive: `sart(pj, flip=True, **kw)` / `sart_device(pj)`, an iterative convertor (ordered-subset SART on the projector and its
+exact adjoint, include/ipdm_b200.h ipdm_fbp_sart) with `convert`'s contract.  It is not the reference's ART convertor
+(TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector).
 """
 import numpy as np
 import torch
@@ -46,6 +50,21 @@ class FBP:
         x = img.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(img, dtype=np.float32))
         x = x[None] if x.dim() == 2 else x
         out = self.project_device(x.to(self.device), flip).cpu()
+        return out if as_tensor else out.numpy()
+
+    def sart_device(self, pj, flip=True, **kw):
+        """Iterative convertor: [B,2000,912] CUDA line integrals -> [B,512,512] CUDA image by ordered-subset SART (keywords
+        iterations, subsets, relaxation; see engine.FBPPlan.sart), no host copy, current stream."""
+        with torch.cuda.device(self.device):
+            return self._plan.sart(pj.contiguous().float(), flip=flip, **kw)
+
+    def sart(self, pj, flip=True, **kw):
+        """`convert`'s contract with SART instead of FBP: ndarray or Tensor [B,2000,912] / [2000,912] in, the same kind out,
+        [B,512,512] float32 on the host."""
+        as_tensor = isinstance(pj, torch.Tensor)
+        x = pj.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(pj, dtype=np.float32))
+        x = x[None] if x.dim() == 2 else x
+        out = self.sart_device(x.to(self.device), flip, **kw).cpu()
         return out if as_tensor else out.numpy()
 
     def convert(self, pj, flip=True):

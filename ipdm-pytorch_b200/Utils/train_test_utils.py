@@ -9,7 +9,8 @@ drive it unchanged.  Differences, all additive:
   * `progressive_denoiser(..., noise=(proj_tape, img_tape))` injects caller noise for parity runs;
   * `simulate_low_dose` makes low-dose inputs from full-dose images or sinograms on the device, and the
     option of the same name makes `test()` use it instead of reading low-dose files;
-  * between the projection stage, the FBP convertor, the sharpen filter and the image stage the
+  * `convertor="SART"` (ordered-subset SART on the device, `sart_*` options) is a second convertor next to FBP;
+  * between the projection stage, the convertor, the sharpen filter and the image stage the
     data stays on the GPU (the reference crosses to the host three times, SURVEY 3.2);
   * training (`train`, the train branch of `fit`), figures and skimage/piq metrics are out of scope.
 """
@@ -199,9 +200,12 @@ class progressive_domain_denoiser:
         if convertor == "FBP":
             self._fbp = FBP(device=self.opt.device)
             self.convertor = self._fbp.convert
+        elif convertor == "SART":
+            self._fbp = FBP(device=self.opt.device)
+            self.convertor = lambda pj, flip=True: self._fbp.sart(pj, flip, **self._sart_kw())
         else:
             def _unsupported(*a, **k):
-                raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP'; the ART "
+                raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP' and 'SART'; the ART "
                                    "extension TASART2DNSL0.pyd is Windows-only): call update_opt(dict(convertor='FBP'))")
             self.convertor = _unsupported
         self.projection = functools.partial(proj_torch, lut_area=None, betas=None)
@@ -265,17 +269,25 @@ class progressive_domain_denoiser:
                 self._drop_graph()
             self._fbp_cap = int(batch)
 
+    def _sart_kw(self):
+        """The sart_* options, read at call time (update_opt needs no re-init)."""
+        o = self.opt
+        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation)
+
     def _convert_device(self, sino):
-        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan."""
+        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan: SART when opt.convertor is 'SART', FBP otherwise."""
         self._reserve_fbp(sino.shape[0])
         G = 10 if self.opt.clip_proj else 1
         s = sino[:, 0].float()
-        return self._fbp.convert_device(s * G if G != 1 else s)[:, None]
+        s = s * G if G != 1 else s
+        if self.opt.convertor == "SART":
+            return self._fbp.sart_device(s, **self._sart_kw())[:, None]
+        return self._fbp.convert_device(s)[:, None]
 
     def simulate_low_dose(self, fd, dose=None, slice_ids=None):
         """Low-dose inputs at `dose` (default opt.dose) from a full-dose batch: a sinogram [B,1,2000,912] gets the dose-reduction
         noise of the reference's Low_dose_CT_simulate.add_noise; a mu image [B,1,512,512] is forward-projected (FBP geometry,
-        Joseph's method) first.  Returns (ldproj [B,1,2000,912], ldct [B,1,512,512] = FBP of ldproj, no sharpen), both on the
+        Joseph's method) first.  Returns (ldproj [B,1,2000,912], ldct [B,1,512,512] = ldproj through the convertor, no sharpen), both on the
         device.  The noise is drawn in line-integral units from Philox keyed by (a hash of noise_seed, slice id, bin), slice ids
         default to 0..B-1; with clip_proj, sinograms are in the dataset's units (line integrals / 10) on the way in and out."""
         o = self.opt

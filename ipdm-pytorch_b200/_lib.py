@@ -51,6 +51,8 @@ _SIGNATURES = {
     "ipdm_fbp_convert_host": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int]),
     "ipdm_fbp_tables": (ctypes.c_int, [vp, vp, vp, vp, vp]),
     "ipdm_fbp_project": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
+    "ipdm_fbp_project_adjoint": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
+    "ipdm_fbp_sart": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, vp]),
     "ipdm_low_dose_noise": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_size_t, ctypes.c_float, ctypes.c_int, ctypes.c_uint64, vp,
                                            vp]),
     "ipdm_cosine_beta_schedule": (ctypes.c_int, [ctypes.c_int, ctypes.c_double, c_double_p]),

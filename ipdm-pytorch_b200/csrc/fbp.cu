@@ -120,20 +120,6 @@ fbp_filter_kernel(const float* __restrict__ sino, float* __restrict__ q, const f
 constexpr int BP_VC = 16;                         // views per staged chunk
 template <int PX> struct BpCfg { static constexpr int SEG = PX == 4 ? 160 : (PX == 2 ? 128 : 112); };
 
-__device__ __forceinline__ float atan_small(float t) {
-    // atan(t) = t * P(t^2), |t| <= 0.62, |err| < 1.3e-10 in exact arithmetic (fit: see DESIGN.md)
-    const float z = t * t;
-    float p = -2.018183097e-02f;
-    p = fmaf(p, z, 5.469628051e-02f);
-    p = fmaf(p, z, -8.460120857e-02f);
-    p = fmaf(p, z, 1.100626141e-01f);
-    p = fmaf(p, z, -1.427598149e-01f);
-    p = fmaf(p, z, 1.999954879e-01f);
-    p = fmaf(p, z, -3.333332539e-01f);
-    p = fmaf(p, z, 1.0f);
-    return t * p;
-}
-
 // detector coordinate u = (atan(s/c) - nda[0])/da + 0.5 and 1/L^2 for one pixel and view
 __device__ __forceinline__ void ray_coords(float x, float y, float cs, float sn, float inv_da, float u_off,
                                            float& u, float& w) {
@@ -288,6 +274,7 @@ extern "C" int ipdm_fbp_plan_create(ipdm_fbp_plan** out, int max_batch) {
 extern "C" int ipdm_fbp_plan_destroy(ipdm_fbp_plan* p) {
     if (!p) return IPDM_OK;
     cudaFree(p->d_wcos); cudaFree(p->d_htap); cudaFree(p->d_cs); cudaFree(p->d_ray); cudaFree(p->d_work);
+    release_sart(p);
     delete p;
     return IPDM_OK;
 }

@@ -9,11 +9,13 @@
 // Discrete model: Joseph's method.  Along the dominant axis of the ray (columns j when |cos phi| >= |sin phi|, rows i otherwise)
 // one sample per column / row m, at the fractional index u(m) = u0 + (m - 255.5) g of the other axis, linear between the two pixel
 // centres that straddle it (weights in fp32, no texture filtering), times the step dx / |cos| (or |sin|); fp32 accumulation in
-// ascending m.  The test suite's C checker restates the same sums in fp64.
+// ascending m.  The test suite's C checker restates the same sums in fp64.  The per-ray setup (u0, g, dominant axis, step) is
+// joseph_ray in fbp_plan.cuh, which the adjoint (sart.cu) evaluates too.
 //
 // Kernel 1  project_transpose_kernel  one 32 x 32 tile per CTA: T[b][j][i] = native[b][i][j].  Column-major rays then read T
 //           along a row, so a warp of adjacent detectors reads adjacent words of one row in either case (1 MB per slice).
-// Kernel 2  fbp_project_kernel        one thread per ray, a warp on 32 adjacent detectors of one view; each ray only loops over
+// Kernel 2  fbp_project_kernel        one thread per ray (of all views, or of one SART subset), a warp on 32 adjacent detectors
+//           of one view; each ray only loops over
 //           the columns / rows where it is inside the grid.  Bound: gather through L1 (about 0.75 G samples, 2 loads each, per
 //           slice; compulsory HBM bytes 1 MB image + 7.3 MB sinogram per slice).
 // Kernel 3  low_dose_noise_kernel     one thread per 4 bins: out = p + sqrt((1-f) e^p (1 + (1+f) Ne e^p / (f N0)) / (f N0)) n,
@@ -26,7 +28,6 @@ namespace ipdm {
 
 constexpr int NV = IPDM_N_VIEWS, ND = IPDM_N_DET, NP = IPDM_N_PIX;
 constexpr int PROJ_THREADS = 256;
-static_assert((NV * ND) % PROJ_THREADS == 0, "one thread per ray, no tail");
 
 __global__ void __launch_bounds__(256) project_transpose_kernel(const float* __restrict__ img, float* __restrict__ t, int flip) {
     __shared__ float tile[32][33];
@@ -61,23 +62,16 @@ __device__ __forceinline__ float joseph_sum(const float* __restrict__ plane, int
     return acc;
 }
 
+// rays of the views v0 + n * vstep, n < nv (all 2000 views: 0, 1, 2000); sino is [B][nv][912]
 __global__ void __launch_bounds__(PROJ_THREADS)
 fbp_project_kernel(const float* __restrict__ img, const float* __restrict__ imgT, float* __restrict__ sino,
-                   const float2* __restrict__ cs_view, const float2* __restrict__ cs_ray, int flip) {
-    const int ray = blockIdx.x * PROJ_THREADS + threadIdx.x;          // v * ND + k
-    const int v = ray / ND, k = ray - v * ND;
+                   const float2* __restrict__ cs_view, const float2* __restrict__ cs_ray, int flip, int v0, int vstep, int nv) {
+    const int ray = blockIdx.x * PROJ_THREADS + threadIdx.x;          // n * ND + k
+    if (ray >= nv * ND) return;
+    const int n = ray / ND, k = ray - n * ND;
     const size_t b = blockIdx.y;
-    constexpr float dx = 42.0f / 512.0f;
-    const float2 th = __ldg(cs_view + v), al = __ldg(cs_ray + k);
-    const float cphi = fmaf(th.x, al.x, th.y * al.y);                // cos(theta - alpha)
-    const float sphi = fmaf(th.y, al.x, -th.x * al.y);               // sin(theta - alpha)
-    const float p = (59.5f / dx) * al.y;                              // D sin(alpha) in pixel units
-    const bool xmajor = fabsf(cphi) >= fabsf(sphi);
-    // x-major: row index r(j) = 255.5 - p / cos + (j - 255.5) tan;  y-major: column index c(i) = 255.5 + p / sin + (i - 255.5) cot
-    const float a = xmajor ? cphi : sphi, o = xmajor ? sphi : cphi;
-    const float ra = 1.0f / a;
-    const float u0 = xmajor ? fmaf(-p, ra, 255.5f) : fmaf(p, ra, 255.5f);
-    const float g = o * ra;
+    const JosephRay r = joseph_ray(__ldg(cs_view + v0 + n * vstep), __ldg(cs_ray + k));
+    const float u0 = r.u0, g = r.g;
     // columns / rows where -1 <= u < 512 (the only ones with a non-zero tap), one of slack on either side
     int m_lo = 0, m_hi = NP - 1;
     if (fabsf(g) > 1e-6f) {
@@ -86,10 +80,10 @@ fbp_project_kernel(const float* __restrict__ img, const float* __restrict__ imgT
         m_hi = min(NP - 1, (int)ceilf(fminf(fmaxf(ma, mb), (float)NP + 1.0f)) + 1);
     }
     float acc;
-    if (xmajor) acc = joseph_sum<false>(imgT + b * NP * NP, m_lo, m_hi, u0, g);
+    if (r.xmajor) acc = joseph_sum<false>(imgT + b * NP * NP, m_lo, m_hi, u0, g);
     else if (flip) acc = joseph_sum<true>(img + b * NP * NP, m_lo, m_hi, u0, g);
     else acc = joseph_sum<false>(img + b * NP * NP, m_lo, m_hi, u0, g);
-    sino[b * NV * ND + (size_t)v * ND + (flip ? ND - 1 - k : k)] = acc * (dx * fabsf(ra));
+    sino[b * nv * ND + (size_t)n * ND + (flip ? ND - 1 - k : k)] = acc * r.scale;
 }
 
 __global__ void __launch_bounds__(256)
@@ -118,21 +112,25 @@ low_dose_noise_kernel(const float* sino, const float* __restrict__ noise, float*
     }
 }
 
+int launch_project(ipdm_fbp_plan* p, const float* img, float* sino, int batch, int flip, int v0, int vstep, int nv, cudaStream_t st) {
+    IPDM_CHECK(ensure_workspace(p, batch));
+    project_transpose_kernel<<<dim3(NP / 32, NP / 32, batch), dim3(32, 8), 0, st>>>(img, p->d_work, flip);
+    count_launch();
+    IPDM_CHECK_LAUNCH();
+    fbp_project_kernel<<<dim3(ceil_div((long long)nv * ND, PROJ_THREADS), batch), PROJ_THREADS, 0, st>>>(img, p->d_work, sino, p->d_cs,
+                                                                                                          p->d_ray, flip, v0, vstep, nv);
+    count_launch();
+    IPDM_CHECK_LAUNCH();
+    return IPDM_OK;
+}
+
 }  // namespace ipdm
 
 using namespace ipdm;
 
 extern "C" int ipdm_fbp_project(ipdm_fbp_plan* p, const float* img, float* sino, int batch, int flip, void* stream) {
     IPDM_REQUIRE(p && img && sino && batch > 0 && batch <= 65535, "ipdm_fbp_project: bad arguments");
-    IPDM_CHECK(ensure_workspace(p, batch));
-    cudaStream_t st = (cudaStream_t)stream;
-    project_transpose_kernel<<<dim3(NP / 32, NP / 32, batch), dim3(32, 8), 0, st>>>(img, p->d_work, flip);
-    count_launch();
-    IPDM_CHECK_LAUNCH();
-    fbp_project_kernel<<<dim3(NV * ND / PROJ_THREADS, batch), PROJ_THREADS, 0, st>>>(img, p->d_work, sino, p->d_cs, p->d_ray, flip);
-    count_launch();
-    IPDM_CHECK_LAUNCH();
-    return IPDM_OK;
+    return launch_project(p, img, sino, batch, flip, 0, 1, NV, (cudaStream_t)stream);
 }
 
 extern "C" int ipdm_low_dose_noise(const float* sino, const float* noise, float* out, int batch, size_t n_per_slice, float dose,

@@ -14,6 +14,7 @@ from . import _lib
 from ._lib import GuidedParams, UNetConfig, check
 
 N_VIEWS, N_DET, N_PIX = 2000, 912, 512
+SART_DEFAULTS = dict(iterations=5, subsets=100, relaxation=1.0)     # the sart_* options of Config/default_config.py
 PRECISIONS = {"tf32": 0, "bf16": 1, "fp32": 2}
 
 
@@ -132,6 +133,48 @@ class FBPPlan:
         if tuple(out.shape) != (b, N_VIEWS, N_DET):
             raise ValueError(f"out must be [{b},{N_VIEWS},{N_DET}], got {tuple(out.shape)}")
         check(_lib.lib().ipdm_fbp_project(self._h, _dev(img, "img"), _dev(out, "out"), b, int(bool(flip)), _stream()), "ipdm_fbp_project")
+        return out
+
+    def _image_out(self, out, b, like):
+        out = torch.empty(b, N_PIX, N_PIX, device=like.device, dtype=torch.float32) if out is None else out
+        if tuple(out.shape) != (b, N_PIX, N_PIX):
+            raise ValueError(f"out must be [{b},{N_PIX},{N_PIX}], got {tuple(out.shape)}")
+        return out
+
+    def project_adjoint(self, sino, flip=True, out=None):
+        """Exact adjoint (transpose) of `project`: [B,2000,912] device -> [B,512,512] device, the same weights and flip frames, so
+        <project(x), y> = <x, project_adjoint(y)> up to fp32 rounding.  Deterministic and slice by slice."""
+        self._check_sino(sino)
+        b = sino.shape[0]
+        out = self._image_out(out, b, sino)
+        check(_lib.lib().ipdm_fbp_project_adjoint(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), _stream()),
+              "ipdm_fbp_project_adjoint")
+        return out
+
+    @staticmethod
+    def check_sart_args(iterations, subsets, relaxation):
+        """ValueError unless iterations >= 1, subsets divides 2000 and 0 < relaxation < 2; returns them as (int, int, float)."""
+        if isinstance(iterations, bool) or int(iterations) != iterations or iterations < 1:
+            raise ValueError(f"SART iterations must be an integer >= 1, got {iterations!r}")
+        if isinstance(subsets, bool) or int(subsets) != subsets or not 1 <= subsets <= N_VIEWS or N_VIEWS % int(subsets):
+            raise ValueError(f"SART subsets must be an integer dividing {N_VIEWS}, got {subsets!r}")
+        if not 0.0 < float(relaxation) < 2.0:
+            raise ValueError(f"SART relaxation must be in (0, 2), got {relaxation!r}")
+        return int(iterations), int(subsets), float(relaxation)
+
+    def sart(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"],
+             relaxation=SART_DEFAULTS["relaxation"], out=None):
+        """Ordered-subset SART (see include/ipdm_b200.h ipdm_fbp_sart): line integrals [B,2000,912] device -> mu image [B,512,512]
+        device in the frame of `forward` for the same flip.  The first call for a subset count builds the plan's tables and
+        synchronises; later calls allocate nothing (CUDA-graph safe)."""
+        self._check_sino(sino)
+        iterations, subsets, relaxation = self.check_sart_args(iterations, subsets, relaxation)
+        b = sino.shape[0]
+        out = self._image_out(out, b, sino)
+        if out.data_ptr() == sino.data_ptr():
+            raise ValueError("out must not alias sino")
+        check(_lib.lib().ipdm_fbp_sart(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
+                                       ctypes.c_float(relaxation), _stream()), "ipdm_fbp_sart")
         return out
 
     def tables(self):
