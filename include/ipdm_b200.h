@@ -99,7 +99,7 @@ int ipdm_fbp_project(ipdm_fbp_plan* plan, const float* img_dev, float* sino_dev,
  * projector applies (the same weights, bit for bit) and the same flip frames.  Deterministic (no atomics), slice by slice. */
 int ipdm_fbp_project_adjoint(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, void* stream);
 /* Ordered-subset SART convertor (replaces the SART core of the reference's Windows-only ART convertor TASART2DNSL0.pyd,
- * correction_kernel / update_kernel; not its NSL0-TV step): line integrals sino [B,2000,912] -> mu image img [B,512,512], frames
+ * correction_kernel / update_kernel; not its NSL0 step, see ipdm_fbp_sart_tv for a TV-regularised variant): line integrals sino [B,2000,912] -> mu image img [B,512,512], frames
  * as for ipdm_fbp_forward.  Subset s = views v with v mod S = s, S = subsets dividing 2000; a sweep visits s_n = n p mod S,
  * p the integer in [1, S) coprime to S closest to 0.382 S (smaller on a tie; 1 when S <= 2).  x0 = 0; per subset
  * r = (b - A_s x) / R (0 where R = A 1 is 0), x <- max(0, x + relaxation * A_s^T r / C_s) where C_s = A_s^T 1 > 0.
@@ -108,6 +108,20 @@ int ipdm_fbp_project_adjoint(ipdm_fbp_plan* plan, const float* sino_dev, float* 
  * nothing and do not synchronise. */
 int ipdm_fbp_sart(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets,
                   float relaxation, void* stream);
+/* SART-TV (ASD-POCS with a fixed step fraction; not the reference's NSL0 formula): ipdm_fbp_sart from x0 = 0 (init_fbp = 0) or
+ * x0 = max(0, ipdm_fbp_forward(sino)) (init_fbp = 1, unsharpened; then the first subset is projected too), and after every sweep
+ * ntv steps of normalised steepest descent on TV_eps(x) = sum sqrt(dx^2 + dy^2 + tv_eps^2) (forward differences in the native
+ * frame, 0 where they would leave the image): x <- max(0, x - t g / |g|_2), g = grad TV_eps(x), per slice, t = tv_alpha |x - x_prev|_2
+ * with x_prev the iterate before the sweep (no change where |g| = 0).  Norms are fp64 sums in a fixed order: results are
+ * bit-identical from run to run and per slice, flip = 1 gives the column mirror of flip = 0 bit for bit, and ntv = 0 with
+ * init_fbp = 0 is ipdm_fbp_sart bit for bit.  Checks of ipdm_fbp_sart plus ntv >= 0, tv_alpha and tv_eps finite and > 0,
+ * init_fbp in {0, 1}, img 16-byte aligned.  The TV workspace (2 images + 4.1 KB per slice) lives in the plan; after the first
+ * call of a shape a call allocates nothing and does not synchronise. */
+int ipdm_fbp_sart_tv(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets,
+                     float relaxation, int ntv, float tv_alpha, float tv_eps, int init_fbp, void* stream);
+/* The TV steps alone, in place on img [B,512,512] (frame flip): `steps` steps of length `step` (the same for every slice) as in
+ * ipdm_fbp_sart_tv.  steps >= 0, step finite and >= 0, eps finite and > 0, img 16-byte aligned. */
+int ipdm_fbp_tv_descent(ipdm_fbp_plan* plan, float* img_dev, int batch, int flip, int steps, float step, float eps, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Diffusion schedule.  Replaces Model/model.py: cosine_beta_schedule :366-372 and

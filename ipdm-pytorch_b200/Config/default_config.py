@@ -8,7 +8,9 @@ the reference's "no key names ..." line otherwise.  Additive keys of this build:
 ("tf32" | "fp32" | "bf16"), `noise_seed`, `cuda_graph`, `simulate_low_dose` (the test loop makes
 its low-dose inputs from the full-dose data at `dose` instead of reading them) and the settings of
 the `convertor="SART"` convertor, `sart_iterations` (sweeps), `sart_subsets` (S, divides 2000) and
-`sart_relaxation` (lambda in (0, 2)); their defaults reproduce the reference.
+`sart_relaxation` (lambda in (0, 2)); their defaults reproduce the reference.  The reference's `ntv` is read by
+`convertor="SART"`: the number of TV steps after every sweep (SART-TV; 0, the default, is plain SART), with `tv_alpha` (step
+fraction of the sweep's change), `tv_eps` (TV smoothing, 1/cm) and `sart_init` ("zero" | "fbp": the start image).
 """
 import argparse
 import json
@@ -52,7 +54,7 @@ _FLAGS = [
     # additive (B200 build)
     ("precision", str, "tf32", None), ("noise_seed", int, 0, None), ("cuda_graph", bool, False, None),
     ("simulate_low_dose", bool, False, None), ("sart_iterations", int, 5, None), ("sart_subsets", int, 100, None),
-    ("sart_relaxation", float, 1.0, None),
+    ("sart_relaxation", float, 1.0, None), ("tv_alpha", float, 0.2, None), ("tv_eps", float, 1e-4, None), ("sart_init", str, "zero", None),
 ]
 
 

@@ -11,8 +11,9 @@ Additive: `project(img, flip=True)` / `project_device(img)`, the forward project
 for sample.
 
 Additive: `sart(pj, flip=True, **kw)` / `sart_device(pj)`, an iterative convertor (ordered-subset SART on the projector and its
-exact adjoint, include/ipdm_b200.h ipdm_fbp_sart) with `convert`'s contract.  It is not the reference's ART convertor
-(TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector).
+exact adjoint, include/ipdm_b200.h ipdm_fbp_sart; with ntv > 0 or init="fbp" SART-TV, ipdm_fbp_sart_tv) with `convert`'s
+contract.  It is not the reference's ART convertor (TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector):
+its TV steps are ASD-POCS steps on a smoothed isotropic TV, not the NSL0 formula.
 """
 import numpy as np
 import torch
@@ -54,7 +55,8 @@ class FBP:
 
     def sart_device(self, pj, flip=True, **kw):
         """Iterative convertor: [B,2000,912] CUDA line integrals -> [B,512,512] CUDA image by ordered-subset SART (keywords
-        iterations, subsets, relaxation; see engine.FBPPlan.sart), no host copy, current stream."""
+        iterations, subsets, relaxation, and ntv, tv_alpha, tv_eps, init of SART-TV; see engine.FBPPlan.sart), no host copy,
+        current stream."""
         with torch.cuda.device(self.device):
             return self._plan.sart(pj.contiguous().float(), flip=flip, **kw)
 

@@ -9,7 +9,8 @@ drive it unchanged.  Differences, all additive:
   * `progressive_denoiser(..., noise=(proj_tape, img_tape))` injects caller noise for parity runs;
   * `simulate_low_dose` makes low-dose inputs from full-dose images or sinograms on the device, and the
     option of the same name makes `test()` use it instead of reading low-dose files;
-  * `convertor="SART"` (ordered-subset SART on the device, `sart_*` options) is a second convertor next to FBP;
+  * `convertor="SART"` (ordered-subset SART on the device, `sart_*` options; SART-TV with `ntv` > 0) is a second convertor
+    next to FBP;
   * between the projection stage, the convertor, the sharpen filter and the image stage the
     data stays on the GPU (the reference crosses to the host three times, SURVEY 3.2);
   * training (`train`, the train branch of `fit`), figures and skimage/piq metrics are out of scope.
@@ -270,9 +271,11 @@ class progressive_domain_denoiser:
             self._fbp_cap = int(batch)
 
     def _sart_kw(self):
-        """The sart_* options, read at call time (update_opt needs no re-init)."""
+        """The sart_* options and the TV options of SART-TV (ntv, tv_alpha, tv_eps, sart_init), read at call time (update_opt needs
+        no re-init)."""
         o = self.opt
-        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation)
+        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation, ntv=o.ntv, tv_alpha=o.tv_alpha,
+                    tv_eps=o.tv_eps, init=o.sart_init)
 
     def _convert_device(self, sino):
         """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan: SART when opt.convertor is 'SART', FBP otherwise."""

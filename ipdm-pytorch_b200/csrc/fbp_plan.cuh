@@ -1,5 +1,5 @@
-// The FBP plan (geometry tables + workspace), shared by the convertor (fbp.cu), the forward projector (project.cu) and its
-// adjoint / SART (sart.cu), and the device helpers more than one of them evaluates.
+// The FBP plan (geometry tables + workspace), shared by the convertor (fbp.cu), the forward projector (project.cu), its
+// adjoint / SART (sart.cu) and the TV steps (tv.cu), and the device helpers more than one of them evaluates.
 #pragma once
 #include "common.cuh"
 
@@ -34,6 +34,9 @@ struct ipdm_fbp_plan {
     std::map<int, float*> colsum;
     float* d_sart = nullptr;
     size_t sart_bytes = 0;
+    // TV steps (tv.cu): g and x_prev [tv_cap][512][512] f32, per-tile partial sums [tv_cap][2][256] and step lengths [tv_cap] f64
+    void* d_tv = nullptr;
+    int tv_cap = 0;
 };
 
 namespace ipdm {
@@ -41,6 +44,14 @@ namespace ipdm {
 int ensure_workspace(ipdm_fbp_plan* plan, int batch);
 // frees the SART tables and workspace (sart.cu)
 void release_sart(ipdm_fbp_plan* plan);
+// grows the TV workspace to `batch` slices (it is never shrunk); frees it (tv.cu)
+int ensure_tv_workspace(ipdm_fbp_plan* plan, int batch);
+void release_tv(ipdm_fbp_plan* plan);
+// the workspace's x_prev images [tv_cap][512][512], the iterate before a SART sweep
+float* tv_prev(ipdm_fbp_plan* plan);
+// `steps` TV steps on img [B][512][512] (column-flipped iff flip), in place.  sweep: the step length is alpha_or_step times
+// |img - tv_prev| of each slice, taken at the first step; otherwise alpha_or_step itself (tv.cu)
+int launch_tv(ipdm_fbp_plan* p, float* img, int batch, int flip, int steps, bool sweep, double alpha_or_step, float eps, cudaStream_t st);
 // transpose + Joseph projection of the views v0 + n * vstep, n < nv: img [B][512][512] -> sino [B][nv][912] (project.cu)
 int launch_project(ipdm_fbp_plan* p, const float* img, float* sino, int batch, int flip, int v0, int vstep, int nv, cudaStream_t st);
 

@@ -1,6 +1,7 @@
 // Iterative convertor for sm_100a: the exact adjoint of the forward projector (project.cu) and ordered-subset SART around the
-// projector / adjoint pair, in the FBP plan's geometry and flip frames.  A new convertor, not a port of the reference's
-// Windows-only TASART2DNSL0.pyd (whose projector is an area-integral model and whose NSL0-TV step is not restated here).
+// projector / adjoint pair, in the FBP plan's geometry and flip frames, optionally started from the FBP image and regularised by
+// TV steps between the sweeps (SART-TV, tv.cu).  A new convertor, not a port of the reference's Windows-only TASART2DNSL0.pyd:
+// its area-integral projector and its NSL0 formula are not ported (the TV steps here are ASD-POCS on a smoothed isotropic TV).
 //
 // A is the fp32 matrix ipdm_fbp_project applies: ray (v, k) samples column / row m of its dominant axis at u = joseph_u(m) and
 // puts the weights 1 - w on pixel floor(u) and w on floor(u) + 1 of the other axis (w = u - floor(u)), times the ray's step.
@@ -14,9 +15,12 @@
 //           SART: the staged value is the ray's residual (b - A_s x) / R (0 where R = 0), and the epilogue applies
 //           x <- max(0, x + lambda * A_s^T r / C_s) (pixels with C_s = 0 keep x).  Bound: FP32 issue on the candidate loop.
 // Kernel 2  fill_kernel                the all-ones image / sinogram the tables R = A 1 and C_s = A_s^T 1 are computed from.
+// Kernel 3  clamp_nonneg_kernel        x0 = max(0, FBP) of the FBP start.
+// SART-TV: before every sweep the iterate is copied to the TV workspace's x_prev, after it ntv TV steps run (launch_tv).
 #include "fbp_plan.cuh"
 
 #include <cmath>
+#include <cstdint>
 #include <numeric>
 
 namespace ipdm {
@@ -146,6 +150,15 @@ __global__ void fill_kernel(float* p, float v, int n) {
     if (i < n) p[i] = v;
 }
 
+__global__ void clamp_nonneg_kernel(float4* p, size_t n) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        float4 v = p[i];
+        v.x = fmaxf(0.f, v.x); v.y = fmaxf(0.f, v.y); v.z = fmaxf(0.f, v.z); v.w = fmaxf(0.f, v.w);
+        p[i] = v;
+    }
+}
+
 template <bool SART>
 static int launch_adjoint(ipdm_fbp_plan* p, const float* y, const float* psub, const float* colsum, float* img, int batch, int flip, int v0,
                           int vstep, int nv, float lambda, cudaStream_t st) {
@@ -207,26 +220,15 @@ void release_sart(ipdm_fbp_plan* p) {
     p->d_rowsum = p->d_sart = nullptr;
     p->colsum.clear();
     p->sart_bytes = 0;
+    release_tv(p);
 }
 
-}  // namespace ipdm
-
-using namespace ipdm;
-
-extern "C" int ipdm_fbp_project_adjoint(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, void* stream) {
-    IPDM_REQUIRE(p && sino && img && batch > 0 && batch <= 65535, "ipdm_fbp_project_adjoint: bad arguments");
-    return launch_adjoint<false>(p, sino, nullptr, nullptr, img, batch, flip, 0, 1, NV, 0.f, (cudaStream_t)stream);
-}
-
-extern "C" int ipdm_fbp_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
-                             float relaxation, void* stream) {
-    IPDM_REQUIRE(p && sino && img && sino != img && batch > 0 && batch <= 65535, "ipdm_fbp_sart: bad arguments");
-    IPDM_REQUIRE(iterations >= 1, "ipdm_fbp_sart: iterations must be >= 1, got %d", iterations);
-    IPDM_REQUIRE(subsets >= 1 && subsets <= NV && NV % subsets == 0, "ipdm_fbp_sart: subsets must divide %d, got %d", NV, subsets);
-    IPDM_REQUIRE(relaxation > 0.f && relaxation < 2.f, "ipdm_fbp_sart: relaxation must be in (0, 2), got %g", (double)relaxation);
-    cudaStream_t st = (cudaStream_t)stream;
+// SART (ntv = 0) or SART-TV, from x0 = 0 (init_fbp = 0) or x0 = max(0, FBP(sino)) (init_fbp = 1); arguments checked by the callers
+static int run_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets, float relaxation,
+                    int ntv, float tv_alpha, float tv_eps, int init_fbp, cudaStream_t st) {
     IPDM_CHECK(ensure_sart_tables(p, subsets, st));
     IPDM_CHECK(ensure_workspace(p, batch));                                    // the projector's transposed iterates
+    if (ntv > 0) IPDM_CHECK(ensure_tv_workspace(p, batch));                    // g, x_prev and the partial sums of the TV steps
     const int nv = NV / subsets;
     const size_t need = (size_t)batch * nv * ND * sizeof(float);               // A_s x of one subset
     if (need > p->sart_bytes) {
@@ -238,17 +240,61 @@ extern "C" int ipdm_fbp_sart(ipdm_fbp_plan* p, const float* sino, float* img, in
     }
     const float* colsum = p->colsum[subsets];
     const int step = sart_visit_step(subsets);
-    IPDM_CHECK_CUDA(cudaMemsetAsync(img, 0, (size_t)batch * NP * NP * sizeof(float), st));       // x0 = 0
+    const size_t img_bytes = (size_t)batch * NP * NP * sizeof(float);
+    if (init_fbp) {                                                            // x0 = max(0, FBP(sino)), unsharpened
+        IPDM_CHECK(ipdm_fbp_forward(p, sino, img, batch, flip, st));
+        const size_t n4 = (size_t)batch * NP * NP / 4;
+        clamp_nonneg_kernel<<<ceil_div((long long)n4, 256), 256, 0, st>>>(reinterpret_cast<float4*>(img), n4);
+        count_launch();
+        IPDM_CHECK_LAUNCH();
+    } else {
+        IPDM_CHECK_CUDA(cudaMemsetAsync(img, 0, img_bytes, st));              // x0 = 0
+    }
     for (int it = 0; it < iterations; ++it) {
+        if (ntv > 0) IPDM_CHECK_CUDA(cudaMemcpyAsync(tv_prev(p), img, img_bytes, cudaMemcpyDeviceToDevice, st));
         for (int n = 0; n < subsets; ++n) {
             const int s = (int)((long long)n * step % subsets);
-            const float* proj = nullptr;                                       // A_s x0 = 0: the first subset needs no projection
-            if (it > 0 || n > 0) {
+            const float* proj = nullptr;                                       // A_s x0 = 0: the first subset from 0 needs no projection
+            if (init_fbp || it > 0 || n > 0) {
                 IPDM_CHECK(launch_project(p, img, p->d_sart, batch, flip, s, subsets, nv, st));
                 proj = p->d_sart;
             }
             IPDM_CHECK(launch_adjoint<true>(p, sino, proj, colsum + (size_t)s * NP * NP, img, batch, flip, s, subsets, nv, relaxation, st));
         }
+        if (ntv > 0) IPDM_CHECK(launch_tv(p, img, batch, flip, ntv, true, (double)tv_alpha, tv_eps, st));
     }
     return IPDM_OK;
+}
+
+}  // namespace ipdm
+
+using namespace ipdm;
+
+extern "C" int ipdm_fbp_project_adjoint(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, void* stream) {
+    IPDM_REQUIRE(p && sino && img && batch > 0 && batch <= 65535, "ipdm_fbp_project_adjoint: bad arguments");
+    return launch_adjoint<false>(p, sino, nullptr, nullptr, img, batch, flip, 0, 1, NV, 0.f, (cudaStream_t)stream);
+}
+
+// the argument checks both SART entries share
+#define SART_CHECK_ARGS(fn)                                                                                                       \
+    IPDM_REQUIRE(p && sino && img && sino != img && batch > 0 && batch <= 65535, fn ": bad arguments");                          \
+    IPDM_REQUIRE(iterations >= 1, fn ": iterations must be >= 1, got %d", iterations);                                          \
+    IPDM_REQUIRE(subsets >= 1 && subsets <= NV && NV % subsets == 0, fn ": subsets must divide %d, got %d", NV, subsets);       \
+    IPDM_REQUIRE(relaxation > 0.f && relaxation < 2.f, fn ": relaxation must be in (0, 2), got %g", (double)relaxation)
+
+extern "C" int ipdm_fbp_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
+                             float relaxation, void* stream) {
+    SART_CHECK_ARGS("ipdm_fbp_sart");
+    return run_sart(p, sino, img, batch, flip, iterations, subsets, relaxation, 0, 0.f, 0.f, 0, (cudaStream_t)stream);
+}
+
+extern "C" int ipdm_fbp_sart_tv(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
+                                float relaxation, int ntv, float tv_alpha, float tv_eps, int init_fbp, void* stream) {
+    SART_CHECK_ARGS("ipdm_fbp_sart_tv");
+    IPDM_REQUIRE(ntv >= 0, "ipdm_fbp_sart_tv: ntv must be >= 0, got %d", ntv);
+    IPDM_REQUIRE(std::isfinite(tv_alpha) && tv_alpha > 0.f, "ipdm_fbp_sart_tv: tv_alpha must be finite and > 0, got %g", (double)tv_alpha);
+    IPDM_REQUIRE(std::isfinite(tv_eps) && tv_eps > 0.f, "ipdm_fbp_sart_tv: tv_eps must be finite and > 0, got %g", (double)tv_eps);
+    IPDM_REQUIRE(init_fbp == 0 || init_fbp == 1, "ipdm_fbp_sart_tv: init_fbp must be 0 or 1, got %d", init_fbp);
+    IPDM_REQUIRE(((uintptr_t)img & 15) == 0, "ipdm_fbp_sart_tv: img must be 16-byte aligned");
+    return run_sart(p, sino, img, batch, flip, iterations, subsets, relaxation, ntv, tv_alpha, tv_eps, init_fbp, (cudaStream_t)stream);
 }

@@ -15,6 +15,9 @@ from ._lib import GuidedParams, UNetConfig, check
 
 N_VIEWS, N_DET, N_PIX = 2000, 912, 512
 SART_DEFAULTS = dict(iterations=5, subsets=100, relaxation=1.0)     # the sart_* options of Config/default_config.py
+# the TV options of SART-TV (ntv, tv_alpha, tv_eps, sart_init of Config/default_config.py); ntv = 0 with the zero start is plain SART
+SART_TV_DEFAULTS = dict(ntv=0, tv_alpha=0.2, tv_eps=1e-4, init="zero")
+SART_INITS = ("zero", "fbp")
 PRECISIONS = {"tf32": 0, "bf16": 1, "fp32": 2}
 
 
@@ -152,30 +155,70 @@ class FBPPlan:
         return out
 
     @staticmethod
-    def check_sart_args(iterations, subsets, relaxation):
-        """ValueError unless iterations >= 1, subsets divides 2000 and 0 < relaxation < 2; returns them as (int, int, float)."""
+    def check_tv_args(ntv=SART_TV_DEFAULTS["ntv"], tv_alpha=SART_TV_DEFAULTS["tv_alpha"], tv_eps=SART_TV_DEFAULTS["tv_eps"],
+                      init=SART_TV_DEFAULTS["init"]):
+        """ValueError unless ntv is an integer >= 0, tv_alpha and tv_eps are finite and > 0 and init is "zero" or "fbp"; returns
+        them as (int, float, float, str)."""
+        if isinstance(ntv, bool) or not isinstance(ntv, (int, np.integer)) or ntv < 0:
+            raise ValueError(f"SART-TV ntv must be an integer >= 0, got {ntv!r}")
+        for name, v in (("tv_alpha", tv_alpha), ("tv_eps", tv_eps)):
+            if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or not (math.isfinite(v) and v > 0):
+                raise ValueError(f"SART-TV {name} must be finite and > 0, got {v!r}")
+        if init not in SART_INITS:
+            raise ValueError(f"SART init must be one of {SART_INITS}, got {init!r}")
+        return int(ntv), float(tv_alpha), float(tv_eps), str(init)
+
+    @staticmethod
+    def check_sart_args(iterations, subsets, relaxation, **tv):
+        """ValueError unless iterations >= 1, subsets divides 2000 and 0 < relaxation < 2 (and the keywords of `check_tv_args`, when
+        given, pass it); returns (iterations, subsets, relaxation) as (int, int, float)."""
         if isinstance(iterations, bool) or int(iterations) != iterations or iterations < 1:
             raise ValueError(f"SART iterations must be an integer >= 1, got {iterations!r}")
         if isinstance(subsets, bool) or int(subsets) != subsets or not 1 <= subsets <= N_VIEWS or N_VIEWS % int(subsets):
             raise ValueError(f"SART subsets must be an integer dividing {N_VIEWS}, got {subsets!r}")
         if not 0.0 < float(relaxation) < 2.0:
             raise ValueError(f"SART relaxation must be in (0, 2), got {relaxation!r}")
+        FBPPlan.check_tv_args(**tv)
         return int(iterations), int(subsets), float(relaxation)
 
     def sart(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"],
-             relaxation=SART_DEFAULTS["relaxation"], out=None):
+             relaxation=SART_DEFAULTS["relaxation"], out=None, ntv=SART_TV_DEFAULTS["ntv"], tv_alpha=SART_TV_DEFAULTS["tv_alpha"],
+             tv_eps=SART_TV_DEFAULTS["tv_eps"], init=SART_TV_DEFAULTS["init"]):
         """Ordered-subset SART (see include/ipdm_b200.h ipdm_fbp_sart): line integrals [B,2000,912] device -> mu image [B,512,512]
-        device in the frame of `forward` for the same flip.  The first call for a subset count builds the plan's tables and
-        synchronises; later calls allocate nothing (CUDA-graph safe)."""
+        device in the frame of `forward` for the same flip.  With ntv > 0 or init="fbp" it is SART-TV (ipdm_fbp_sart_tv): the
+        start is max(0, forward(sino)) for init="fbp", and every sweep is followed by ntv TV steps of length tv_alpha |x - x_prev|
+        (tv_eps in 1/cm smooths the TV).  The first call for a subset count builds the plan's tables and synchronises; later calls
+        allocate nothing (CUDA-graph safe)."""
         self._check_sino(sino)
         iterations, subsets, relaxation = self.check_sart_args(iterations, subsets, relaxation)
+        ntv, tv_alpha, tv_eps, init = self.check_tv_args(ntv, tv_alpha, tv_eps, init)
         b = sino.shape[0]
         out = self._image_out(out, b, sino)
         if out.data_ptr() == sino.data_ptr():
             raise ValueError("out must not alias sino")
-        check(_lib.lib().ipdm_fbp_sart(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
-                                       ctypes.c_float(relaxation), _stream()), "ipdm_fbp_sart")
+        if ntv == 0 and init == "zero":
+            check(_lib.lib().ipdm_fbp_sart(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
+                                           ctypes.c_float(relaxation), _stream()), "ipdm_fbp_sart")
+        else:
+            check(_lib.lib().ipdm_fbp_sart_tv(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
+                                              ctypes.c_float(relaxation), ntv, ctypes.c_float(tv_alpha), ctypes.c_float(tv_eps),
+                                              int(init == "fbp"), _stream()), "ipdm_fbp_sart_tv")
         return out
+
+    def tv_descent(self, img, steps, step, eps=SART_TV_DEFAULTS["tv_eps"], flip=True):
+        """`steps` TV steps of length `step` (the same for every slice) on a [B,512,512] device image, in place: the regulariser of
+        SART-TV on its own (include/ipdm_b200.h ipdm_fbp_tv_descent).  Returns img."""
+        if img.dim() != 3 or tuple(img.shape[1:]) != (N_PIX, N_PIX):
+            raise ValueError(f"image must be [B,{N_PIX},{N_PIX}], got {tuple(img.shape)}")
+        if isinstance(steps, bool) or int(steps) != steps or steps < 0:
+            raise ValueError(f"TV steps must be an integer >= 0, got {steps!r}")
+        if not (math.isfinite(step) and step >= 0):
+            raise ValueError(f"TV step must be finite and >= 0, got {step!r}")
+        if not (math.isfinite(eps) and eps > 0):
+            raise ValueError(f"TV eps must be finite and > 0, got {eps!r}")
+        check(_lib.lib().ipdm_fbp_tv_descent(self._h, _dev(img, "img"), img.shape[0], int(bool(flip)), int(steps), ctypes.c_float(step),
+                                             ctypes.c_float(eps), _stream()), "ipdm_fbp_tv_descent")
+        return img
 
     def tables(self):
         theta = np.empty(N_VIEWS, np.float64)

@@ -1,9 +1,11 @@
 """Timing of the iterative convertor: python tools/bench_sart.py [batch ...]  (default 16 64).
 
-CUDA events around ipdm_fbp_project_adjoint and ipdm_fbp_sart (default options) after a warm-up of the same shape, which also
+CUDA events around ipdm_fbp_project_adjoint, ipdm_fbp_sart (default options), one TV step (ipdm_fbp_tv_descent) and SART-TV at
+the recommended setting (ipdm_fbp_sart_tv, ntv = 20, tv_alpha = 0.2, FBP start) after a warm-up of the same shape, which also
 builds SART's geometry tables.  Each timed call reads and writes buffers of its own, rotated so that one round of them exceeds the
 126 MB L2: inputs come from HBM, not from the previous call's cache lines.  Weight updates are counted from the geometry: the
-non-zero entries of A (Joseph taps inside the grid), which the adjoint applies once each.
+non-zero entries of A (Joseph taps inside the grid), which the adjoint applies once each.  The TV step's rate is taken on its
+compulsory bytes, 16 per pixel: x read and written, g written and read.
 """
 import os
 import sys
@@ -18,6 +20,8 @@ from bench_project import L2_BYTES, card, timed
 from ipdm_pytorch_b200 import engine, synthetic as S
 
 NV, ND, NP = engine.N_VIEWS, engine.N_DET, engine.N_PIX
+SART_TV = dict(ntv=20, tv_alpha=0.2, init="fbp")           # the recommended SART-TV setting (DESIGN 8)
+TV_BYTES_PER_PIXEL = 16
 
 
 def entries_per_slice():
@@ -60,10 +64,19 @@ def main():
         print(f"| adjoint (A^T y) | {b} | {ms:.3f} | {ms / b:.3f} | {n_upd * b / ms / 1e6:.1f} |")
         ms = timed(lambda k: plan.project(imgs[k], out=sinos[k]), n_sets, iters)
         print(f"| projector (A x), for reference | {b} | {ms:.3f} | {ms / b:.3f} | {n_upd * b / ms / 1e6:.1f} |")
-        ms = timed(lambda k: plan.sart(sinos[k], out=imgs[k], **d), n_sets, max(3, 64 // b))
-        print(f"| SART, {d['iterations']} sweeps x {d['subsets']} subsets | {b} | {ms:.3f} | {ms / b:.3f} | "
+        ms_sart = timed(lambda k: plan.sart(sinos[k], out=imgs[k], **d), n_sets, max(3, 64 // b))
+        print(f"| SART, {d['iterations']} sweeps x {d['subsets']} subsets | {b} | {ms_sart:.3f} | {ms_sart / b:.3f} | "
+              f"{2 * d['iterations'] * n_upd * b / ms_sart / 1e6:.1f} |")
+        ms = timed(lambda k: plan.sart(sinos[k], out=imgs[k], **d, **SART_TV), n_sets, max(3, 64 // b))
+        print(f"| SART-TV {SART_TV}: {ms / ms_sart - 1:+.1%} over SART | {b} | {ms:.3f} | {ms / b:.3f} | "
               f"{2 * d['iterations'] * n_upd * b / ms / 1e6:.1f} |")
         del sinos, imgs
+        n_img = max(2, -(-2 * L2_BYTES // (4 * b * NP * NP)))
+        xs = [torch.rand(b, NP, NP, device=dev) for _ in range(n_img)]
+        ms = timed(lambda k: plan.tv_descent(xs[k], 1, 1e-4), n_img, max(50, 4000 // b))
+        print(f"| one TV step (gradient + update): {TV_BYTES_PER_PIXEL * b * NP * NP / ms / 1e6:.0f} GB/s on its compulsory bytes "
+              f"| {b} | {ms:.4f} | {ms / b:.4f} | - |")
+        del xs
         torch.cuda.empty_cache()
 
 
