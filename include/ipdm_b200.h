@@ -122,6 +122,27 @@ int ipdm_fbp_sart_tv(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev,
 /* The TV steps alone, in place on img [B,512,512] (frame flip): `steps` steps of length `step` (the same for every slice) as in
  * ipdm_fbp_sart_tv.  steps >= 0, step finite and >= 0, eps finite and > 0, img 16-byte aligned. */
 int ipdm_fbp_tv_descent(ipdm_fbp_plan* plan, float* img_dev, int batch, int flip, int steps, float step, float eps, void* stream);
+/* Penalised weighted least squares (PWLS) solved by ordered-subset separable quadratic surrogates (OS-SQS; Erdogan & Fessler 1999):
+ * line integrals sino [B,2000,912] -> mu image img [B,512,512], frames as for ipdm_fbp_forward.  Minimises
+ * Phi(x) = 1/2 sum_i w_i ([A x]_i - b_i)^2 + beta R(x), x >= 0, A the matrix of ipdm_fbp_project, b = sino, with the weights
+ * w_i = 1 / sigma^2(max(b_i, 0)), sigma^2(p) = e^p / (f N0) (1 + Ne e^p / (f N0)), f = dose, N0 = 1.4e5, Ne = 5.8 (the variance of
+ * a measurement at dose f, as ipdm_low_dose_noise simulates it), computed from b in fp32, and the hyperbola penalty of
+ * ipdm_fbp_pwls_penalty.  D^L = A^T (w o A 1) once per call; subsets and visit order of ipdm_fbp_sart; per subset
+ * x <- max(0, x + (S A_s^T (w_s o (b_s - A_s x)) - beta grad R(x)) / (D^L + beta d^R(x))) (x kept where the denominator is 0).
+ * x0 = 0 (init_fbp = 0) or max(0, ipdm_fbp_forward(sino)) (init_fbp = 1).  Checks of ipdm_fbp_sart (without relaxation) plus dose
+ * in (0, 1], beta finite and >= 0, delta (1/cm) finite and > 0, init_fbp in {0, 1}, img 16-byte aligned.  No atomics: bit-identical
+ * from run to run and per slice, flip = 1 gives the column mirror of flip = 0.  The first call builds R = A 1 and synchronises;
+ * the workspace (3 images per slice) lives in the plan; after the first call of a shape a call allocates nothing and does not
+ * synchronise. */
+int ipdm_fbp_pwls(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets, float dose,
+                  float beta, float delta, int init_fbp, void* stream);
+/* The PWLS penalty alone: grad R and the SQS curvature d^R of every slice of img [B,512,512] (frame flip), into grad / curv
+ * [B,512,512] (the same frame).  R(x) = sum_j sum_{k in N+(j)} kappa_jk psi(x_j - x_k), N+ = right, down, down-left, down-right in
+ * the native frame, kappa = 1 (edge) or 1/sqrt(2) (diagonal), psi(t) = delta^2 (sqrt(1 + (t / delta)^2) - 1);
+ * grad R_j = sum over the 8 neighbours of kappa psi'(x_j - x_k), d^R_j = 2 sum of kappa / sqrt(1 + ((x_j - x_k) / delta)^2).
+ * delta finite and > 0; grad, curv and img distinct. */
+int ipdm_fbp_pwls_penalty(ipdm_fbp_plan* plan, const float* img_dev, float* grad_dev, float* curv_dev, int batch, int flip, float delta,
+                          void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Diffusion schedule.  Replaces Model/model.py: cosine_beta_schedule :366-372 and

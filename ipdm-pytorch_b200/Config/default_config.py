@@ -11,6 +11,9 @@ the `convertor="SART"` convertor, `sart_iterations` (sweeps), `sart_subsets` (S,
 `sart_relaxation` (lambda in (0, 2)); their defaults reproduce the reference.  The reference's `ntv` is read by
 `convertor="SART"`: the number of TV steps after every sweep (SART-TV; 0, the default, is plain SART), with `tv_alpha` (step
 fraction of the sweep's change), `tv_eps` (TV smoothing, 1/cm) and `sart_init` ("zero" | "fbp": the start image).
+`convertor="PWLS"` (penalised weighted least squares by ordered-subset SQS) reads `sart_iterations`, `sart_subsets`, `sart_init`
+and `dose` (the weights are the rays' inverse variances at that dose) and its own `pwls_beta` (penalty weight) and `pwls_delta`
+(edge scale of the hyperbola penalty, 1/cm); it ignores `sart_relaxation` and the TV options.
 """
 import argparse
 import json
@@ -55,6 +58,7 @@ _FLAGS = [
     ("precision", str, "tf32", None), ("noise_seed", int, 0, None), ("cuda_graph", bool, False, None),
     ("simulate_low_dose", bool, False, None), ("sart_iterations", int, 5, None), ("sart_subsets", int, 100, None),
     ("sart_relaxation", float, 1.0, None), ("tv_alpha", float, 0.2, None), ("tv_eps", float, 1e-4, None), ("sart_init", str, "zero", None),
+    ("pwls_beta", float, 1e6, None), ("pwls_delta", float, 0.0002, None),
 ]
 
 

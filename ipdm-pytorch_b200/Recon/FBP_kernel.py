@@ -14,6 +14,9 @@ Additive: `sart(pj, flip=True, **kw)` / `sart_device(pj)`, an iterative converto
 exact adjoint, include/ipdm_b200.h ipdm_fbp_sart; with ntv > 0 or init="fbp" SART-TV, ipdm_fbp_sart_tv) with `convert`'s
 contract.  It is not the reference's ART convertor (TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector):
 its TV steps are ASD-POCS steps on a smoothed isotropic TV, not the NSL0 formula.
+
+Additive: `pwls(pj, flip=True, **kw)` / `pwls_device(pj)`, a statistically weighted iterative convertor (penalised weighted
+least squares with dose-aware weights, solved by ordered-subset SQS, include/ipdm_b200.h ipdm_fbp_pwls) with `convert`'s contract.
 """
 import numpy as np
 import torch
@@ -67,6 +70,21 @@ class FBP:
         x = pj.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(pj, dtype=np.float32))
         x = x[None] if x.dim() == 2 else x
         out = self.sart_device(x.to(self.device), flip, **kw).cpu()
+        return out if as_tensor else out.numpy()
+
+    def pwls_device(self, pj, flip=True, **kw):
+        """Statistically weighted convertor: [B,2000,912] CUDA line integrals -> [B,512,512] CUDA image by PWLS / OS-SQS (keywords
+        iterations, subsets, dose, beta, delta, init; see engine.FBPPlan.pwls), no host copy, current stream."""
+        with torch.cuda.device(self.device):
+            return self._plan.pwls(pj.contiguous().float(), flip=flip, **kw)
+
+    def pwls(self, pj, flip=True, **kw):
+        """`convert`'s contract with PWLS instead of FBP: ndarray or Tensor [B,2000,912] / [2000,912] in, the same kind out,
+        [B,512,512] float32 on the host."""
+        as_tensor = isinstance(pj, torch.Tensor)
+        x = pj.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(pj, dtype=np.float32))
+        x = x[None] if x.dim() == 2 else x
+        out = self.pwls_device(x.to(self.device), flip, **kw).cpu()
         return out if as_tensor else out.numpy()
 
     def convert(self, pj, flip=True):

@@ -11,6 +11,10 @@ drive it unchanged.  Differences, all additive:
     option of the same name makes `test()` use it instead of reading low-dose files;
   * `convertor="SART"` (ordered-subset SART on the device, `sart_*` options; SART-TV with `ntv` > 0) is a second convertor
     next to FBP;
+  * `convertor="PWLS"` (penalised weighted least squares by ordered-subset SQS on the device, `pwls_*` options) is a third.  Its
+    weights are the inverse variances of the rays at `dose`, i.e. they assume the sinogram has dose-f statistics: that holds for
+    the low-dose input (and for `simulate_low_dose`, which converts at the dose it simulated); for the projection stage's
+    denoised output they are a relative reliability per ray, not exact inverse variances;
   * between the projection stage, the convertor, the sharpen filter and the image stage the
     data stays on the GPU (the reference crosses to the host three times, SURVEY 3.2);
   * training (`train`, the train branch of `fit`), figures and skimage/piq metrics are out of scope.
@@ -204,9 +208,12 @@ class progressive_domain_denoiser:
         elif convertor == "SART":
             self._fbp = FBP(device=self.opt.device)
             self.convertor = lambda pj, flip=True: self._fbp.sart(pj, flip, **self._sart_kw())
+        elif convertor == "PWLS":
+            self._fbp = FBP(device=self.opt.device)
+            self.convertor = lambda pj, flip=True: self._fbp.pwls(pj, flip, **self._pwls_kw())
         else:
             def _unsupported(*a, **k):
-                raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP' and 'SART'; the ART "
+                raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP', 'SART' and 'PWLS'; the ART "
                                    "extension TASART2DNSL0.pyd is Windows-only): call update_opt(dict(convertor='FBP'))")
             self.convertor = _unsupported
         self.projection = functools.partial(proj_torch, lut_area=None, betas=None)
@@ -277,21 +284,31 @@ class progressive_domain_denoiser:
         return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation, ntv=o.ntv, tv_alpha=o.tv_alpha,
                     tv_eps=o.tv_eps, init=o.sart_init)
 
-    def _convert_device(self, sino):
-        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan: SART when opt.convertor is 'SART', FBP otherwise."""
+    def _pwls_kw(self, dose=None):
+        """The options convertor="PWLS" reads (sart_iterations, sart_subsets, sart_init, pwls_beta, pwls_delta and the data's dose,
+        opt.dose unless given), at call time."""
+        o = self.opt
+        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, dose=o.dose if dose is None else dose, beta=o.pwls_beta,
+                    delta=o.pwls_delta, init=o.sart_init)
+
+    def _convert_device(self, sino, dose=None):
+        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan: SART when opt.convertor is 'SART', PWLS (weights at
+        `dose`, default opt.dose) when it is 'PWLS', FBP otherwise."""
         self._reserve_fbp(sino.shape[0])
         G = 10 if self.opt.clip_proj else 1
         s = sino[:, 0].float()
         s = s * G if G != 1 else s
         if self.opt.convertor == "SART":
             return self._fbp.sart_device(s, **self._sart_kw())[:, None]
+        if self.opt.convertor == "PWLS":
+            return self._fbp.pwls_device(s, **self._pwls_kw(dose))[:, None]
         return self._fbp.convert_device(s)[:, None]
 
     def simulate_low_dose(self, fd, dose=None, slice_ids=None):
         """Low-dose inputs at `dose` (default opt.dose) from a full-dose batch: a sinogram [B,1,2000,912] gets the dose-reduction
         noise of the reference's Low_dose_CT_simulate.add_noise; a mu image [B,1,512,512] is forward-projected (FBP geometry,
         Joseph's method) first.  Returns (ldproj [B,1,2000,912], ldct [B,1,512,512] = ldproj through the convertor, no sharpen), both on the
-        device.  The noise is drawn in line-integral units from Philox keyed by (a hash of noise_seed, slice id, bin), slice ids
+        device; convertor="PWLS" weights ldproj at the dose it was simulated at.  The noise is drawn in line-integral units from Philox keyed by (a hash of noise_seed, slice id, bin), slice ids
         default to 0..B-1; with clip_proj, sinograms are in the dataset's units (line integrals / 10) on the way in and out."""
         o = self.opt
         fd = fd.to(o.device).float()
@@ -305,9 +322,10 @@ class progressive_domain_denoiser:
             sino = fd[:, 0] * G                                                # always a fresh buffer: the noise is added in place
         else:
             raise ValueError(f"simulate_low_dose: expected [B,1,2000,912] or [B,1,512,512], got {tuple(fd.shape)}")
-        _eng.low_dose_noise(sino, o.dose if dose is None else dose, seed=self._stage_seed(3), slice_ids=slice_ids, clip=True, out=sino)
+        dose = o.dose if dose is None else dose
+        _eng.low_dose_noise(sino, dose, seed=self._stage_seed(3), slice_ids=slice_ids, clip=True, out=sino)
         ldproj = (sino / G if G != 1 else sino)[:, None]
-        return ldproj, self._convert_device(ldproj)
+        return ldproj, self._convert_device(ldproj, dose)
 
     def _img_stage(self, x, noise=None, noise_strength=None):
         o = self.opt

@@ -56,6 +56,9 @@ _SIGNATURES = {
     "ipdm_fbp_sart_tv": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int,
                                         ctypes.c_float, ctypes.c_float, ctypes.c_int, vp]),
     "ipdm_fbp_tv_descent": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_float, vp]),
+    "ipdm_fbp_pwls": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_float,
+                                     ctypes.c_float, ctypes.c_int, vp]),
+    "ipdm_fbp_pwls_penalty": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_float, vp]),
     "ipdm_low_dose_noise": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_size_t, ctypes.c_float, ctypes.c_int, ctypes.c_uint64, vp,
                                            vp]),
     "ipdm_cosine_beta_schedule": (ctypes.c_int, [ctypes.c_int, ctypes.c_double, c_double_p]),

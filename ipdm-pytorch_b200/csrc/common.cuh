@@ -41,6 +41,10 @@ const char* last_error();
 
 constexpr int kNumSMs = 148;
 
+// photon statistics of the dose-reduction noise (project.cu) and of the PWLS weights (sart.cu): N0 incident photons per ray at
+// full dose, Ne electronic-noise variance (the constants of the reference's Utils/Low_dose_CT_simulate.py add_noise)
+constexpr double kDoseN0 = 1.4e5, kDoseNe = 5.8;
+
 inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 // kernel launch counter (bench.py reports it as gpu_launches)

@@ -1,5 +1,6 @@
 // The FBP plan (geometry tables + workspace), shared by the convertor (fbp.cu), the forward projector (project.cu), its
-// adjoint / SART (sart.cu) and the TV steps (tv.cu), and the device helpers more than one of them evaluates.
+// adjoint / SART / PWLS (sart.cu), the TV steps (tv.cu) and the PWLS penalty (pwls.cu), and the device helpers more than one of
+// them evaluates.
 #pragma once
 #include "common.cuh"
 
@@ -37,6 +38,9 @@ struct ipdm_fbp_plan {
     // TV steps (tv.cu): g and x_prev [tv_cap][512][512] f32, per-tile partial sums [tv_cap][2][256] and step lengths [tv_cap] f64
     void* d_tv = nullptr;
     int tv_cap = 0;
+    // PWLS (pwls.cu): D^L, grad R and d^R [pwls_cap][512][512] f32 each
+    float* d_pwls = nullptr;
+    int pwls_cap = 0;
 };
 
 namespace ipdm {
@@ -52,6 +56,15 @@ float* tv_prev(ipdm_fbp_plan* plan);
 // `steps` TV steps on img [B][512][512] (column-flipped iff flip), in place.  sweep: the step length is alpha_or_step times
 // |img - tv_prev| of each slice, taken at the first step; otherwise alpha_or_step itself (tv.cu)
 int launch_tv(ipdm_fbp_plan* p, float* img, int batch, int flip, int steps, bool sweep, double alpha_or_step, float eps, cudaStream_t st);
+// grows the PWLS workspace to `batch` slices (it is never shrunk); frees it; its D^L, grad R and d^R planes [pwls_cap][512][512]
+// (pwls.cu)
+int ensure_pwls_workspace(ipdm_fbp_plan* plan, int batch);
+void release_pwls(ipdm_fbp_plan* plan);
+float* pwls_dl(ipdm_fbp_plan* plan);
+float* pwls_grad(ipdm_fbp_plan* plan);
+float* pwls_curv(ipdm_fbp_plan* plan);
+// grad R and d^R of the hyperbola penalty of img [B][512][512] (column-flipped iff flip), in the same frame (pwls.cu)
+int launch_pwls_penalty(const float* img, float* grad, float* curv, int batch, int flip, float delta, cudaStream_t st);
 // transpose + Joseph projection of the views v0 + n * vstep, n < nv: img [B][512][512] -> sino [B][nv][912] (project.cu)
 int launch_project(ipdm_fbp_plan* p, const float* img, float* sino, int batch, int flip, int v0, int vstep, int nv, cudaStream_t st);
 

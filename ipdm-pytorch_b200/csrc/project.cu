@@ -138,7 +138,7 @@ extern "C" int ipdm_low_dose_noise(const float* sino, const float* noise, float*
     IPDM_REQUIRE(sino && out && batch > 0 && batch <= 65535 && n_per_slice > 0 && n_per_slice / 4 < (1ull << 32),
                  "ipdm_low_dose_noise: bad arguments");
     IPDM_REQUIRE(dose > 0.f && dose <= 1.f, "ipdm_low_dose_noise: dose must be in (0, 1], got %g", (double)dose);
-    const double f = dose, ne = 5.8, n0 = 1.4e5;
+    const double f = dose, ne = kDoseNe, n0 = kDoseN0;
     const float ka = (float)((1.0 - f) / (f * n0)), kc = (float)((1.0 + f) * ne / (f * n0));
     const size_t quads = (n_per_slice + 3) / 4;
     low_dose_noise_kernel<<<dim3(ceil_div((long long)quads, 256), batch), 256, 0, (cudaStream_t)stream>>>(

@@ -1,12 +1,13 @@
-// Iterative convertor for sm_100a: the exact adjoint of the forward projector (project.cu) and ordered-subset SART around the
+// Iterative convertors for sm_100a: the exact adjoint of the forward projector (project.cu), ordered-subset SART around the
 // projector / adjoint pair, in the FBP plan's geometry and flip frames, optionally started from the FBP image and regularised by
-// TV steps between the sweeps (SART-TV, tv.cu).  A new convertor, not a port of the reference's Windows-only TASART2DNSL0.pyd:
+// TV steps between the sweeps (SART-TV, tv.cu), and penalised weighted least squares solved by ordered-subset SQS (PWLS, with the
+// penalty of pwls.cu).  A new convertor, not a port of the reference's Windows-only TASART2DNSL0.pyd:
 // its area-integral projector and its NSL0 formula are not ported (the TV steps here are ASD-POCS on a smoothed isotropic TV).
 //
 // A is the fp32 matrix ipdm_fbp_project applies: ray (v, k) samples column / row m of its dominant axis at u = joseph_u(m) and
 // puts the weights 1 - w on pixel floor(u) and w on floor(u) + 1 of the other axis (w = u - floor(u)), times the ray's step.
 //
-// Kernel 1  fbp_adjoint_kernel<SART>  pixel-driven gather, one CTA per 32 x 32 pixel tile and slice, ascending views.  Per
+// Kernel 1  fbp_adjoint_kernel<MODE>  pixel-driven gather, one CTA per 32 x 32 pixel tile and slice, ascending views.  Per
 //           16-view chunk the CTA stages, for the detector segment its tile can touch, each ray's (u0, g, step * value, axis)
 //           in shared memory; the ray setup is joseph_ray, so every weight is the projector's own fp32 weight.  A pixel then
 //           tries the rays within dx / (L da) + 1 pitches of its own fan angle (L its distance from the source): a ray passes
@@ -14,9 +15,13 @@
 //           floor and a compare.  No atomics: each output pixel is one thread's sum in a fixed order.
 //           SART: the staged value is the ray's residual (b - A_s x) / R (0 where R = 0), and the epilogue applies
 //           x <- max(0, x + lambda * A_s^T r / C_s) (pixels with C_s = 0 keep x).  Bound: FP32 issue on the candidate loop.
+//           PWLS: DENOM stages w(b) R and writes D^L = A^T (w o R); SQS stages w(b) (b - A_s x) and the epilogue applies
+//           x <- max(0, x + (S A_s^T(...) - beta grad R) / (D^L + beta d^R)) (pixels with a zero denominator keep x), with
+//           w(b) = 1 / sigma^2(max(b, 0)) computed from b in fp32 (no weight sinogram is stored).
 // Kernel 2  fill_kernel                the all-ones image / sinogram the tables R = A 1 and C_s = A_s^T 1 are computed from.
 // Kernel 3  clamp_nonneg_kernel        x0 = max(0, FBP) of the FBP start.
 // SART-TV: before every sweep the iterate is copied to the TV workspace's x_prev, after it ntv TV steps run (launch_tv).
+// PWLS: D^L once per call, then per subset transpose, projection, penalty (launch_pwls_penalty) and the SQS adjoint.
 #include "fbp_plan.cuh"
 
 #include <cmath>
@@ -32,6 +37,23 @@ constexpr int ADJ_RPT = 4;                 // pixel rows per thread
 constexpr int ADJ_TH = 8 * ADJ_RPT;        // tile rows
 constexpr float DXP = 42.0f / 512.0f;
 
+// what fbp_adjoint_kernel stages per ray and does with the sums
+enum AdjMode { ADJ_PLAIN, ADJ_SART, ADJ_DENOM, ADJ_SQS };
+
+// the PWLS operands of the DENOM and SQS modes: wk = 1 / (dose N0); dl, grad, curv [B][512][512] in the image's frame (SQS)
+struct PwlsArgs {
+    const float* dl = nullptr;
+    const float* grad = nullptr;
+    const float* curv = nullptr;
+    float wk = 0.f, beta = 0.f;
+};
+
+// w = 1 / sigma^2(max(b, 0)), sigma^2(p) = q (1 + Ne q), q = e^p / (dose N0): the inverse variance of a measurement at the dose
+__device__ __forceinline__ float pwls_weight(float b, float wk) {
+    const float q = expf(fmaxf(b, 0.f)) * wk;
+    return 1.0f / (q * fmaf((float)kDoseNe, q, 1.0f));
+}
+
 // continuous ray index kc of the pixel centre (x, y) in view cs = (cos theta, sin theta), and the half width hw of its candidate
 // window: dx / (L da) pitches plus one of slack (the rounding of kc is about 1e-4 pitch)
 __device__ __forceinline__ void pixel_window(float x, float y, float2 cs, float inv_da, float k_off, float& kc, float& hw) {
@@ -41,37 +63,46 @@ __device__ __forceinline__ void pixel_window(float x, float y, float2 cs, float 
     hw = fmaf(DXP * inv_da, rsqrtf(fmaf(s, s, c * c)), 1.0f);
 }
 
-// staged entry of ray (v, k): (u0, g, step * value, xmajor); value = y[v][k'] (plain adjoint) or the SART residual of the ray,
-// k' = k in the sinogram's frame.  yb / pb / R are per-slice; pb (the subset projection, row n) is null when x = 0.
-template <bool SART>
+// staged entry of ray (v, k): (u0, g, step * value, xmajor); value = y[v][k'] (plain adjoint), the SART residual of the ray,
+// w(b) R (DENOM) or w(b) (b - A_s x) (SQS), k' = k in the sinogram's frame.  yb / pb / R are per-slice; pb (the subset
+// projection, row n) is null when x = 0.
+template <int MODE>
 __device__ __forceinline__ float4 adj_entry(const float* __restrict__ yb, const float* __restrict__ pb, const float* __restrict__ R,
                                             const float2* __restrict__ cs_view, const float2* __restrict__ cs_ray, int v, int n, int k,
-                                            int flip) {
+                                            int flip, float wk) {
     const JosephRay r = joseph_ray(__ldg(cs_view + v), __ldg(cs_ray + k));
     const int kk = flip ? ND - 1 - k : k;
     float val = __ldg(yb + (size_t)v * ND + kk);
-    if (SART) {
+    if (MODE == ADJ_SART) {
         const float rs = __ldg(R + (size_t)v * ND + k);
         if (pb) val -= __ldg(pb + (size_t)n * ND + kk);
         val = rs > 0.f ? val / rs : 0.f;
+    } else if (MODE == ADJ_DENOM) {
+        val = pwls_weight(val, wk) * __ldg(R + (size_t)v * ND + k);
+    } else if (MODE == ADJ_SQS) {
+        const float w = pwls_weight(val, wk);
+        if (pb) val -= __ldg(pb + (size_t)n * ND + kk);
+        val *= w;
     }
     return make_float4(r.u0, r.g, r.scale * val, r.xmajor ? 1.f : 0.f);
 }
 
 // the same, out of line: a ray outside the staged segment (kept off the candidate loop's registers)
-template <bool SART>
+template <int MODE>
 __device__ __noinline__ float4 adj_entry_far(const float* yb, const float* pb, const float* R, const float2* cs_view, const float2* cs_ray,
-                                             int v, int n, int k, int flip) {
-    return adj_entry<SART>(yb, pb, R, cs_view, cs_ray, v, n, k, flip);
+                                             int v, int n, int k, int flip, float wk) {
+    return adj_entry<MODE>(yb, pb, R, cs_view, cs_ray, v, n, k, flip, wk);
 }
 
-// views v0 + n * vstep, n < nv.  y: [B][2000][912] (the sinogram, or b for SART); psub: [B][nv][912] A_s x (SART, may be null);
-// R: [2000][912]; colsum: C_s [512][512] native; img: written (plain) or updated in place (SART), column-flipped iff flip
-template <bool SART>
+// views v0 + n * vstep, n < nv.  y: [B][2000][912] (the sinogram, or b for SART / PWLS); psub: [B][nv][912] A_s x (SART / SQS,
+// may be null); R: [2000][912]; colsum: C_s [512][512] native (SART); img: written (plain, DENOM) or updated in place (SART,
+// SQS), column-flipped iff flip; lambda: the relaxation (SART) or S (SQS)
+template <int MODE>
 __global__ void __launch_bounds__(256)
 fbp_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ psub, const float* __restrict__ R,
                    const float* __restrict__ colsum, float* __restrict__ img, const float2* __restrict__ cs_view,
-                   const float2* __restrict__ cs_ray, int v0, int vstep, int nv, float inv_da, float k_off, float lambda, int flip) {
+                   const float2* __restrict__ cs_ray, int v0, int vstep, int nv, float inv_da, float k_off, float lambda, int flip,
+                   PwlsArgs pw) {
     __shared__ float4 seg[ADJ_VC][ADJ_SEG];
     __shared__ int seg0[ADJ_VC];
     __shared__ float2 scs[ADJ_VC];
@@ -103,7 +134,7 @@ fbp_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ psub, 
         __syncthreads();
         for (int e = tid; e < nvc * ADJ_SEG; e += 256) {
             const int vv = e / ADJ_SEG, o = e - vv * ADJ_SEG;
-            seg[vv][o] = adj_entry<SART>(yb, pb, R, cs_view, cs_ray, v0 + (c0 + vv) * vstep, c0 + vv, seg0[vv] + o, flip);
+            seg[vv][o] = adj_entry<MODE>(yb, pb, R, cs_view, cs_ray, v0 + (c0 + vv) * vstep, c0 + vv, seg0[vv] + o, flip, pw.wk);
         }
         __syncthreads();
         for (int vv = 0; vv < nvc; ++vv) {
@@ -119,7 +150,8 @@ fbp_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ psub, 
                     const int o = k - k0;
                     const float4 e = (unsigned)o < (unsigned)ADJ_SEG
                                          ? seg[vv][o]
-                                         : adj_entry_far<SART>(yb, pb, R, cs_view, cs_ray, v0 + (c0 + vv) * vstep, c0 + vv, k, flip);
+                                         : adj_entry_far<MODE>(yb, pb, R, cs_view, cs_ray, v0 + (c0 + vv) * vstep, c0 + vv, k, flip,
+                                                               pw.wk);
                     const bool xm = e.w != 0.f;
                     const float u = fmaf((float)(xm ? j : i) - 255.5f, e.y, e.x);     // joseph_u at this pixel's column / row
                     const float kf = floorf(u);
@@ -131,16 +163,24 @@ fbp_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ psub, 
             }
         }
     }
-    float* ob = img + (size_t)blockIdx.z * NP * NP;
+    const size_t slice = (size_t)blockIdx.z * NP * NP;
+    float* ob = img + slice;
     const int jo = flip ? NP - 1 - j : j;
 #pragma unroll
     for (int p = 0; p < ADJ_RPT; ++p) {
         const int i = i_base + 8 * p;
-        if (!SART) {
+        if (MODE == ADJ_PLAIN || MODE == ADJ_DENOM) {
             ob[(size_t)i * NP + jo] = acc[p];
-        } else {
+        } else if (MODE == ADJ_SART) {
             const float cs = __ldg(colsum + (size_t)i * NP + j);
             if (cs > 0.f) ob[(size_t)i * NP + jo] = fmaxf(0.f, fmaf(lambda, acc[p] / cs, ob[(size_t)i * NP + jo]));
+        } else {
+            const size_t m = slice + (size_t)i * NP + jo;
+            const float den = fmaf(pw.beta, __ldg(pw.curv + m), __ldg(pw.dl + m));
+            if (den > 0.f) {
+                const float num = fmaf(lambda, acc[p], -pw.beta * __ldg(pw.grad + m));
+                ob[(size_t)i * NP + jo] = fmaxf(0.f, ob[(size_t)i * NP + jo] + num / den);
+            }
         }
     }
 }
@@ -159,12 +199,12 @@ __global__ void clamp_nonneg_kernel(float4* p, size_t n) {
     }
 }
 
-template <bool SART>
+template <int MODE>
 static int launch_adjoint(ipdm_fbp_plan* p, const float* y, const float* psub, const float* colsum, float* img, int batch, int flip, int v0,
-                          int vstep, int nv, float lambda, cudaStream_t st) {
+                          int vstep, int nv, float lambda, cudaStream_t st, const PwlsArgs& pw = PwlsArgs()) {
     const float k_off = (float)(-0.5 - (double)p->host.nda[0] / p->host.da);     // ray k is at fan angle nda[0] + (k + 1/2) da
-    fbp_adjoint_kernel<SART><<<dim3(NP / 32, NP / ADJ_TH, batch), 256, 0, st>>>(y, psub, p->d_rowsum, colsum, img, p->d_cs, p->d_ray, v0,
-                                                                                vstep, nv, p->inv_da, k_off, lambda, flip);
+    fbp_adjoint_kernel<MODE><<<dim3(NP / 32, NP / ADJ_TH, batch), 256, 0, st>>>(y, psub, p->d_rowsum, colsum, img, p->d_cs, p->d_ray, v0,
+                                                                                vstep, nv, p->inv_da, k_off, lambda, flip, pw);
     count_launch();
     IPDM_CHECK_LAUNCH();
     return IPDM_OK;
@@ -181,36 +221,60 @@ static int sart_visit_step(int S) {
     return best;
 }
 
-// R = A 1 (once per plan) and C_s = A_s^T 1 for every subset of S (once per plan and S), in fp32 with the same kernels
-static int ensure_sart_tables(ipdm_fbp_plan* p, int S, cudaStream_t st) {
-    const bool need_r = p->d_rowsum == nullptr, need_c = p->colsum.count(S) == 0;
-    if (!need_r && !need_c) return IPDM_OK;
+// a table build allocates and synchronises, so it cannot run inside a stream capture
+static int require_eager(cudaStream_t st, const char* what) {
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     IPDM_CHECK_CUDA(cudaStreamIsCapturing(st, &cap));
-    IPDM_REQUIRE(cap == cudaStreamCaptureStatusNone,
-                 "ipdm_fbp_sart: the first call with %d subsets builds the plan's tables and cannot be captured; run it once eagerly", S);
-    float* ones = nullptr;
-    IPDM_CHECK_CUDA(cudaMalloc(&ones, (size_t)NV * ND * sizeof(float)));       // all-ones sinogram, and image (its first 512 x 512)
-    int rc = IPDM_OK;
-    fill_kernel<<<ceil_div(NV * ND, 256), 256, 0, st>>>(ones, 1.0f, NV * ND);
+    IPDM_REQUIRE(cap == cudaStreamCaptureStatusNone, "%s cannot be captured; run it once eagerly", what);
+    return IPDM_OK;
+}
+
+// an all-ones sinogram [2000][912]; its first 512 x 512 values serve as the all-ones image
+static int make_ones(float** ones, cudaStream_t st) {
+    IPDM_CHECK_CUDA(cudaMalloc(ones, (size_t)NV * ND * sizeof(float)));
+    fill_kernel<<<ceil_div(NV * ND, 256), 256, 0, st>>>(*ones, 1.0f, NV * ND);
     count_launch();
-    if (cudaGetLastError() != cudaSuccess) rc = IPDM_ERR_CUDA;
-    if (rc == IPDM_OK && need_r) {
-        if (cudaMalloc(&p->d_rowsum, (size_t)NV * ND * sizeof(float)) != cudaSuccess) rc = IPDM_ERR_CUDA;
-        if (rc == IPDM_OK) rc = launch_project(p, ones, p->d_rowsum, 1, 0, 0, 1, NV, st);
-    }
-    if (rc == IPDM_OK && need_c) {
-        float* c = nullptr;
-        if (cudaMalloc(&c, (size_t)S * NP * NP * sizeof(float)) != cudaSuccess) rc = IPDM_ERR_CUDA;
-        for (int s = 0; rc == IPDM_OK && s < S; ++s)
-            rc = launch_adjoint<false>(p, ones, nullptr, nullptr, c + (size_t)s * NP * NP, 1, 0, s, S, NV / S, 0.f, st);
-        if (rc == IPDM_OK) p->colsum[S] = c;
-        else cudaFree(c);
-    }
+    return IPDM_OK;
+}
+
+// ends a table build: waits for it, frees the ones buffer and reports a CUDA failure under fn's name
+static int finish_build(int rc, float* ones, const char* fn, cudaStream_t st) {
+    if (rc == IPDM_OK && cudaGetLastError() != cudaSuccess) rc = IPDM_ERR_CUDA;
     if (cudaStreamSynchronize(st) != cudaSuccess && rc == IPDM_OK) rc = IPDM_ERR_CUDA;
     cudaFree(ones);
-    if (rc == IPDM_ERR_CUDA) set_error("ipdm_fbp_sart: building the tables failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (rc == IPDM_ERR_CUDA) set_error("%s: building the tables failed: %s", fn, cudaGetErrorString(cudaGetLastError()));
     return rc;
+}
+
+// R = A 1, once per plan, in fp32 with the projector; fn names the calling entry in messages
+static int ensure_rowsum(ipdm_fbp_plan* p, const char* fn, cudaStream_t st) {
+    if (p->d_rowsum) return IPDM_OK;
+    char what[96];
+    snprintf(what, sizeof what, "%s: the first call of a plan builds its row sums and", fn);
+    IPDM_CHECK(require_eager(st, what));
+    float* ones = nullptr;
+    IPDM_CHECK(make_ones(&ones, st));
+    int rc = cudaMalloc(&p->d_rowsum, (size_t)NV * ND * sizeof(float)) == cudaSuccess ? IPDM_OK : IPDM_ERR_CUDA;
+    if (rc == IPDM_OK) rc = launch_project(p, ones, p->d_rowsum, 1, 0, 0, 1, NV, st);
+    return finish_build(rc, ones, fn, st);
+}
+
+// R (ensure_rowsum) and C_s = A_s^T 1 for every subset of S (once per plan and S), in fp32 with the same kernels
+static int ensure_sart_tables(ipdm_fbp_plan* p, int S, cudaStream_t st) {
+    IPDM_CHECK(ensure_rowsum(p, "ipdm_fbp_sart", st));
+    if (p->colsum.count(S)) return IPDM_OK;
+    char what[96];
+    snprintf(what, sizeof what, "ipdm_fbp_sart: the first call with %d subsets builds the plan's tables and", S);
+    IPDM_CHECK(require_eager(st, what));
+    float* ones = nullptr;
+    IPDM_CHECK(make_ones(&ones, st));
+    float* c = nullptr;
+    int rc = cudaMalloc(&c, (size_t)S * NP * NP * sizeof(float)) == cudaSuccess ? IPDM_OK : IPDM_ERR_CUDA;
+    for (int s = 0; rc == IPDM_OK && s < S; ++s)
+        rc = launch_adjoint<ADJ_PLAIN>(p, ones, nullptr, nullptr, c + (size_t)s * NP * NP, 1, 0, s, S, NV / S, 0.f, st);
+    if (rc == IPDM_OK) p->colsum[S] = c;
+    else cudaFree(c);
+    return finish_build(rc, ones, "ipdm_fbp_sart", st);
 }
 
 void release_sart(ipdm_fbp_plan* p) {
@@ -221,6 +285,34 @@ void release_sart(ipdm_fbp_plan* p) {
     p->colsum.clear();
     p->sart_bytes = 0;
     release_tv(p);
+    release_pwls(p);
+}
+
+// grows the subset projections A_s x to `batch` slices of nv views (never shrunk)
+static int ensure_subset_buffer(ipdm_fbp_plan* p, int batch, int nv) {
+    const size_t need = (size_t)batch * nv * ND * sizeof(float);
+    if (need > p->sart_bytes) {
+        IPDM_CHECK_CUDA(cudaFree(p->d_sart));
+        p->d_sart = nullptr;
+        p->sart_bytes = 0;
+        IPDM_CHECK_CUDA(cudaMalloc(&p->d_sart, need));
+        p->sart_bytes = need;
+    }
+    return IPDM_OK;
+}
+
+// the start of an iterative convertor: x0 = max(0, FBP(sino)), unsharpened (init_fbp = 1), or x0 = 0
+static int set_start(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int init_fbp, cudaStream_t st) {
+    if (init_fbp) {
+        IPDM_CHECK(ipdm_fbp_forward(p, sino, img, batch, flip, st));
+        const size_t n4 = (size_t)batch * NP * NP / 4;
+        clamp_nonneg_kernel<<<ceil_div((long long)n4, 256), 256, 0, st>>>(reinterpret_cast<float4*>(img), n4);
+        count_launch();
+        IPDM_CHECK_LAUNCH();
+    } else {
+        IPDM_CHECK_CUDA(cudaMemsetAsync(img, 0, (size_t)batch * NP * NP * sizeof(float), st));
+    }
+    return IPDM_OK;
 }
 
 // SART (ntv = 0) or SART-TV, from x0 = 0 (init_fbp = 0) or x0 = max(0, FBP(sino)) (init_fbp = 1); arguments checked by the callers
@@ -230,26 +322,11 @@ static int run_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, 
     IPDM_CHECK(ensure_workspace(p, batch));                                    // the projector's transposed iterates
     if (ntv > 0) IPDM_CHECK(ensure_tv_workspace(p, batch));                    // g, x_prev and the partial sums of the TV steps
     const int nv = NV / subsets;
-    const size_t need = (size_t)batch * nv * ND * sizeof(float);               // A_s x of one subset
-    if (need > p->sart_bytes) {
-        IPDM_CHECK_CUDA(cudaFree(p->d_sart));
-        p->d_sart = nullptr;
-        p->sart_bytes = 0;
-        IPDM_CHECK_CUDA(cudaMalloc(&p->d_sart, need));
-        p->sart_bytes = need;
-    }
+    IPDM_CHECK(ensure_subset_buffer(p, batch, nv));                            // A_s x of one subset
     const float* colsum = p->colsum[subsets];
     const int step = sart_visit_step(subsets);
     const size_t img_bytes = (size_t)batch * NP * NP * sizeof(float);
-    if (init_fbp) {                                                            // x0 = max(0, FBP(sino)), unsharpened
-        IPDM_CHECK(ipdm_fbp_forward(p, sino, img, batch, flip, st));
-        const size_t n4 = (size_t)batch * NP * NP / 4;
-        clamp_nonneg_kernel<<<ceil_div((long long)n4, 256), 256, 0, st>>>(reinterpret_cast<float4*>(img), n4);
-        count_launch();
-        IPDM_CHECK_LAUNCH();
-    } else {
-        IPDM_CHECK_CUDA(cudaMemsetAsync(img, 0, img_bytes, st));              // x0 = 0
-    }
+    IPDM_CHECK(set_start(p, sino, img, batch, flip, init_fbp, st));
     for (int it = 0; it < iterations; ++it) {
         if (ntv > 0) IPDM_CHECK_CUDA(cudaMemcpyAsync(tv_prev(p), img, img_bytes, cudaMemcpyDeviceToDevice, st));
         for (int n = 0; n < subsets; ++n) {
@@ -259,9 +336,42 @@ static int run_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, 
                 IPDM_CHECK(launch_project(p, img, p->d_sart, batch, flip, s, subsets, nv, st));
                 proj = p->d_sart;
             }
-            IPDM_CHECK(launch_adjoint<true>(p, sino, proj, colsum + (size_t)s * NP * NP, img, batch, flip, s, subsets, nv, relaxation, st));
+            IPDM_CHECK(launch_adjoint<ADJ_SART>(p, sino, proj, colsum + (size_t)s * NP * NP, img, batch, flip, s, subsets, nv, relaxation,
+                                                st));
         }
         if (ntv > 0) IPDM_CHECK(launch_tv(p, img, batch, flip, ntv, true, (double)tv_alpha, tv_eps, st));
+    }
+    return IPDM_OK;
+}
+
+// PWLS by OS-SQS (subsets and visit order of SART), from x0 = 0 or max(0, FBP(sino)); arguments checked by the caller
+static int run_pwls(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets, float dose,
+                    float beta, float delta, int init_fbp, cudaStream_t st) {
+    IPDM_CHECK(ensure_rowsum(p, "ipdm_fbp_pwls", st));                         // R, no C_s tables
+    IPDM_CHECK(ensure_workspace(p, batch));
+    IPDM_CHECK(ensure_pwls_workspace(p, batch));                               // D^L, grad R, d^R
+    const int nv = NV / subsets;
+    IPDM_CHECK(ensure_subset_buffer(p, batch, nv));
+    PwlsArgs pw;
+    pw.dl = pwls_dl(p);
+    pw.grad = pwls_grad(p);
+    pw.curv = pwls_curv(p);
+    pw.wk = (float)(1.0 / ((double)dose * kDoseN0));
+    pw.beta = beta;
+    IPDM_CHECK(launch_adjoint<ADJ_DENOM>(p, sino, nullptr, nullptr, pwls_dl(p), batch, flip, 0, 1, NV, 0.f, st, pw));
+    IPDM_CHECK(set_start(p, sino, img, batch, flip, init_fbp, st));
+    const int step = sart_visit_step(subsets);
+    for (int it = 0; it < iterations; ++it) {
+        for (int n = 0; n < subsets; ++n) {
+            const int s = (int)((long long)n * step % subsets);
+            const float* proj = nullptr;                                       // A_s x0 = 0: the first subset from 0 needs no projection
+            if (init_fbp || it > 0 || n > 0) {
+                IPDM_CHECK(launch_project(p, img, p->d_sart, batch, flip, s, subsets, nv, st));
+                proj = p->d_sart;
+            }
+            IPDM_CHECK(launch_pwls_penalty(img, pwls_grad(p), pwls_curv(p), batch, flip, delta, st));
+            IPDM_CHECK(launch_adjoint<ADJ_SQS>(p, sino, proj, nullptr, img, batch, flip, s, subsets, nv, (float)subsets, st, pw));
+        }
     }
     return IPDM_OK;
 }
@@ -272,14 +382,16 @@ using namespace ipdm;
 
 extern "C" int ipdm_fbp_project_adjoint(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, void* stream) {
     IPDM_REQUIRE(p && sino && img && batch > 0 && batch <= 65535, "ipdm_fbp_project_adjoint: bad arguments");
-    return launch_adjoint<false>(p, sino, nullptr, nullptr, img, batch, flip, 0, 1, NV, 0.f, (cudaStream_t)stream);
+    return launch_adjoint<ADJ_PLAIN>(p, sino, nullptr, nullptr, img, batch, flip, 0, 1, NV, 0.f, (cudaStream_t)stream);
 }
 
-// the argument checks both SART entries share
-#define SART_CHECK_ARGS(fn)                                                                                                       \
+// the argument checks all iterative entries share, and the relaxation of the SART entries
+#define ITER_CHECK_ARGS(fn)                                                                                                       \
     IPDM_REQUIRE(p && sino && img && sino != img && batch > 0 && batch <= 65535, fn ": bad arguments");                          \
     IPDM_REQUIRE(iterations >= 1, fn ": iterations must be >= 1, got %d", iterations);                                          \
-    IPDM_REQUIRE(subsets >= 1 && subsets <= NV && NV % subsets == 0, fn ": subsets must divide %d, got %d", NV, subsets);       \
+    IPDM_REQUIRE(subsets >= 1 && subsets <= NV && NV % subsets == 0, fn ": subsets must divide %d, got %d", NV, subsets)
+#define SART_CHECK_ARGS(fn)                                                                                                       \
+    ITER_CHECK_ARGS(fn);                                                                                                          \
     IPDM_REQUIRE(relaxation > 0.f && relaxation < 2.f, fn ": relaxation must be in (0, 2), got %g", (double)relaxation)
 
 extern "C" int ipdm_fbp_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
@@ -297,4 +409,15 @@ extern "C" int ipdm_fbp_sart_tv(ipdm_fbp_plan* p, const float* sino, float* img,
     IPDM_REQUIRE(init_fbp == 0 || init_fbp == 1, "ipdm_fbp_sart_tv: init_fbp must be 0 or 1, got %d", init_fbp);
     IPDM_REQUIRE(((uintptr_t)img & 15) == 0, "ipdm_fbp_sart_tv: img must be 16-byte aligned");
     return run_sart(p, sino, img, batch, flip, iterations, subsets, relaxation, ntv, tv_alpha, tv_eps, init_fbp, (cudaStream_t)stream);
+}
+
+extern "C" int ipdm_fbp_pwls(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets, float dose,
+                             float beta, float delta, int init_fbp, void* stream) {
+    ITER_CHECK_ARGS("ipdm_fbp_pwls");
+    IPDM_REQUIRE(dose > 0.f && dose <= 1.f, "ipdm_fbp_pwls: dose must be in (0, 1], got %g", (double)dose);
+    IPDM_REQUIRE(std::isfinite(beta) && beta >= 0.f, "ipdm_fbp_pwls: beta must be finite and >= 0, got %g", (double)beta);
+    IPDM_REQUIRE(std::isfinite(delta) && delta > 0.f, "ipdm_fbp_pwls: delta must be finite and > 0, got %g", (double)delta);
+    IPDM_REQUIRE(init_fbp == 0 || init_fbp == 1, "ipdm_fbp_pwls: init_fbp must be 0 or 1, got %d", init_fbp);
+    IPDM_REQUIRE(((uintptr_t)img & 15) == 0, "ipdm_fbp_pwls: img must be 16-byte aligned");
+    return run_pwls(p, sino, img, batch, flip, iterations, subsets, dose, beta, delta, init_fbp, (cudaStream_t)stream);
 }

@@ -18,6 +18,8 @@ SART_DEFAULTS = dict(iterations=5, subsets=100, relaxation=1.0)     # the sart_*
 # the TV options of SART-TV (ntv, tv_alpha, tv_eps, sart_init of Config/default_config.py); ntv = 0 with the zero start is plain SART
 SART_TV_DEFAULTS = dict(ntv=0, tv_alpha=0.2, tv_eps=1e-4, init="zero")
 SART_INITS = ("zero", "fbp")
+# the pwls_* options of convertor="PWLS" (pwls_beta, pwls_delta in 1/cm of Config/default_config.py; DESIGN 8 has the study)
+PWLS_DEFAULTS = dict(beta=1e6, delta=0.0002)
 PRECISIONS = {"tf32": 0, "bf16": 1, "fp32": 2}
 
 
@@ -204,6 +206,53 @@ class FBPPlan:
                                               ctypes.c_float(relaxation), ntv, ctypes.c_float(tv_alpha), ctypes.c_float(tv_eps),
                                               int(init == "fbp"), _stream()), "ipdm_fbp_sart_tv")
         return out
+
+    @staticmethod
+    def check_pwls_args(iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=0.25, beta=PWLS_DEFAULTS["beta"],
+                        delta=PWLS_DEFAULTS["delta"], init=SART_TV_DEFAULTS["init"]):
+        """ValueError unless iterations >= 1, subsets divides 2000, 0 < dose <= 1, beta is finite and >= 0, delta is finite and > 0
+        and init is "zero" or "fbp"; returns them as (int, int, float, float, float, str)."""
+        iterations, subsets, _ = FBPPlan.check_sart_args(iterations, subsets, 1.0)
+        real = lambda v: not isinstance(v, bool) and isinstance(v, (int, float, np.integer, np.floating)) and math.isfinite(v)
+        if not (real(dose) and 0.0 < dose <= 1.0):
+            raise ValueError(f"PWLS dose must be in (0, 1], got {dose!r}")
+        if not (real(beta) and beta >= 0):
+            raise ValueError(f"PWLS beta must be finite and >= 0, got {beta!r}")
+        if not (real(delta) and delta > 0):
+            raise ValueError(f"PWLS delta must be finite and > 0, got {delta!r}")
+        if init not in SART_INITS:
+            raise ValueError(f"PWLS init must be one of {SART_INITS}, got {init!r}")
+        return iterations, subsets, float(dose), float(beta), float(delta), str(init)
+
+    def pwls(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=0.25,
+             beta=PWLS_DEFAULTS["beta"], delta=PWLS_DEFAULTS["delta"], init=SART_TV_DEFAULTS["init"], out=None):
+        """Penalised weighted least squares by ordered-subset SQS (see include/ipdm_b200.h ipdm_fbp_pwls): line integrals
+        [B,2000,912] device at dose `dose` -> mu image [B,512,512] device in the frame of `forward` for the same flip.  The weights
+        are the inverse variances of the rays at that dose; beta scales the hyperbola penalty, delta (1/cm) is its edge scale;
+        subsets and sweeps as in `sart`; init="fbp" starts from max(0, forward(sino)).  The first call builds the plan's row sums and
+        synchronises; later calls allocate nothing (CUDA-graph safe)."""
+        self._check_sino(sino)
+        iterations, subsets, dose, beta, delta, init = self.check_pwls_args(iterations, subsets, dose, beta, delta, init)
+        b = sino.shape[0]
+        out = self._image_out(out, b, sino)
+        if out.data_ptr() == sino.data_ptr():
+            raise ValueError("out must not alias sino")
+        check(_lib.lib().ipdm_fbp_pwls(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
+                                       ctypes.c_float(dose), ctypes.c_float(beta), ctypes.c_float(delta), int(init == "fbp"), _stream()),
+              "ipdm_fbp_pwls")
+        return out
+
+    def pwls_penalty(self, img, delta=PWLS_DEFAULTS["delta"], flip=True):
+        """(grad R, d^R) of the PWLS penalty of a [B,512,512] device image, [B,512,512] device each in the image's frame: the
+        regulariser of `pwls` on its own (include/ipdm_b200.h ipdm_fbp_pwls_penalty)."""
+        if img.dim() != 3 or tuple(img.shape[1:]) != (N_PIX, N_PIX):
+            raise ValueError(f"image must be [B,{N_PIX},{N_PIX}], got {tuple(img.shape)}")
+        if not (math.isfinite(delta) and delta > 0):
+            raise ValueError(f"PWLS delta must be finite and > 0, got {delta!r}")
+        grad, curv = torch.empty_like(img), torch.empty_like(img)
+        check(_lib.lib().ipdm_fbp_pwls_penalty(self._h, _dev(img, "img"), _dev(grad, "grad"), _dev(curv, "curv"), img.shape[0],
+                                               int(bool(flip)), ctypes.c_float(delta), _stream()), "ipdm_fbp_pwls_penalty")
+        return grad, curv
 
     def tv_descent(self, img, steps, step, eps=SART_TV_DEFAULTS["tv_eps"], flip=True):
         """`steps` TV steps of length `step` (the same for every slice) on a [B,512,512] device image, in place: the regulariser of

@@ -1,11 +1,13 @@
 """Timing of the iterative convertor: python tools/bench_sart.py [batch ...]  (default 16 64).
 
-CUDA events around ipdm_fbp_project_adjoint, ipdm_fbp_sart (default options), one TV step (ipdm_fbp_tv_descent) and SART-TV at
-the recommended setting (ipdm_fbp_sart_tv, ntv = 20, tv_alpha = 0.2, FBP start) after a warm-up of the same shape, which also
-builds SART's geometry tables.  Each timed call reads and writes buffers of its own, rotated so that one round of them exceeds the
+CUDA events around ipdm_fbp_project_adjoint, ipdm_fbp_sart (default options), one TV step (ipdm_fbp_tv_descent), SART-TV at
+the recommended setting (ipdm_fbp_sart_tv, ntv = 20, tv_alpha = 0.2, FBP start), PWLS at its defaults (ipdm_fbp_pwls, the sweeps
+and subsets of SART, dose 0.25, FBP start) and the PWLS penalty alone (ipdm_fbp_pwls_penalty) after a warm-up of the same shape,
+which also builds SART's geometry tables.  Each timed call reads and writes buffers of its own, rotated so that one round of them exceeds the
 126 MB L2: inputs come from HBM, not from the previous call's cache lines.  Weight updates are counted from the geometry: the
 non-zero entries of A (Joseph taps inside the grid), which the adjoint applies once each.  The TV step's rate is taken on its
-compulsory bytes, 16 per pixel: x read and written, g written and read.
+compulsory bytes, 16 per pixel: x read and written, g written and read; the penalty's on 12 per pixel: x read, grad R and d^R
+written.
 """
 import os
 import sys
@@ -22,6 +24,8 @@ from ipdm_pytorch_b200 import engine, synthetic as S
 NV, ND, NP = engine.N_VIEWS, engine.N_DET, engine.N_PIX
 SART_TV = dict(ntv=20, tv_alpha=0.2, init="fbp")           # the recommended SART-TV setting (DESIGN 8)
 TV_BYTES_PER_PIXEL = 16
+PENALTY_BYTES_PER_PIXEL = 12
+PWLS = dict(dose=0.25, init="fbp", **engine.PWLS_DEFAULTS)
 
 
 def entries_per_slice():
@@ -70,12 +74,19 @@ def main():
         ms = timed(lambda k: plan.sart(sinos[k], out=imgs[k], **d, **SART_TV), n_sets, max(3, 64 // b))
         print(f"| SART-TV {SART_TV}: {ms / ms_sart - 1:+.1%} over SART | {b} | {ms:.3f} | {ms / b:.3f} | "
               f"{2 * d['iterations'] * n_upd * b / ms / 1e6:.1f} |")
+        ms = timed(lambda k: plan.pwls(sinos[k], out=imgs[k], iterations=d["iterations"], subsets=d["subsets"], **PWLS), n_sets,
+                   max(3, 64 // b))
+        print(f"| PWLS {PWLS}: {ms / ms_sart:.2f}x plain SART | {b} | {ms:.3f} | {ms / b:.3f} | "
+              f"{2 * d['iterations'] * n_upd * b / ms / 1e6:.1f} |")
         del sinos, imgs
         n_img = max(2, -(-2 * L2_BYTES // (4 * b * NP * NP)))
         xs = [torch.rand(b, NP, NP, device=dev) for _ in range(n_img)]
         ms = timed(lambda k: plan.tv_descent(xs[k], 1, 1e-4), n_img, max(50, 4000 // b))
         print(f"| one TV step (gradient + update): {TV_BYTES_PER_PIXEL * b * NP * NP / ms / 1e6:.0f} GB/s on its compulsory bytes "
               f"| {b} | {ms:.4f} | {ms / b:.4f} | - |")
+        ms = timed(lambda k: plan.pwls_penalty(xs[k]), n_img, max(50, 4000 // b))
+        print(f"| PWLS penalty (grad R, d^R): {PENALTY_BYTES_PER_PIXEL * b * NP * NP / ms / 1e9:.2f} TB/s on its compulsory bytes "
+              f"| {b} | {ms:.4f} | {ms / b * 1e3:.2f} us | - |")
         del xs
         torch.cuda.empty_cache()
 
