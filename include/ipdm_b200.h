@@ -98,25 +98,22 @@ int ipdm_fbp_project(ipdm_fbp_plan* plan, const float* img_dev, float* sino_dev,
 /* Exact adjoint (transpose) of ipdm_fbp_project: sino [B,2000,912] -> img [B,512,512], img = A^T sino with A the fp32 matrix the
  * projector applies (the same weights, bit for bit) and the same flip frames.  Deterministic (no atomics), slice by slice. */
 int ipdm_fbp_project_adjoint(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, void* stream);
-/* Ordered-subset SART convertor (replaces the SART core of the reference's Windows-only ART convertor TASART2DNSL0.pyd,
- * correction_kernel / update_kernel; not its NSL0 step, see ipdm_fbp_sart_tv for a TV-regularised variant): line integrals sino [B,2000,912] -> mu image img [B,512,512], frames
+/* Ordered-subset SART convertor, optionally regularised by TV steps (SART-TV) and started from the FBP image (replaces the SART
+ * core of the reference's Windows-only ART convertor TASART2DNSL0.pyd, correction_kernel / update_kernel; the TV steps are
+ * ASD-POCS with a fixed step fraction, not its NSL0 formula): line integrals sino [B,2000,912] -> mu image img [B,512,512], frames
  * as for ipdm_fbp_forward.  Subset s = views v with v mod S = s, S = subsets dividing 2000; a sweep visits s_n = n p mod S,
- * p the integer in [1, S) coprime to S closest to 0.382 S (smaller on a tie; 1 when S <= 2).  x0 = 0; per subset
- * r = (b - A_s x) / R (0 where R = A 1 is 0), x <- max(0, x + relaxation * A_s^T r / C_s) where C_s = A_s^T 1 > 0.
- * iterations >= 1 sweeps, 0 < relaxation < 2, img must not alias sino.  R and C_s are built in the plan by the first call
- * for a given S (that call synchronises the stream and cannot be captured); later calls of the same or a smaller shape allocate
- * nothing and do not synchronise. */
-int ipdm_fbp_sart(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets,
-                  float relaxation, void* stream);
-/* SART-TV (ASD-POCS with a fixed step fraction; not the reference's NSL0 formula): ipdm_fbp_sart from x0 = 0 (init_fbp = 0) or
- * x0 = max(0, ipdm_fbp_forward(sino)) (init_fbp = 1, unsharpened; then the first subset is projected too), and after every sweep
- * ntv steps of normalised steepest descent on TV_eps(x) = sum sqrt(dx^2 + dy^2 + tv_eps^2) (forward differences in the native
- * frame, 0 where they would leave the image): x <- max(0, x - t g / |g|_2), g = grad TV_eps(x), per slice, t = tv_alpha |x - x_prev|_2
- * with x_prev the iterate before the sweep (no change where |g| = 0).  Norms are fp64 sums in a fixed order: results are
- * bit-identical from run to run and per slice, flip = 1 gives the column mirror of flip = 0 bit for bit, and ntv = 0 with
- * init_fbp = 0 is ipdm_fbp_sart bit for bit.  Checks of ipdm_fbp_sart plus ntv >= 0, tv_alpha and tv_eps finite and > 0,
- * init_fbp in {0, 1}, img 16-byte aligned.  The TV workspace (2 images + 4.1 KB per slice) lives in the plan; after the first
- * call of a shape a call allocates nothing and does not synchronise. */
+ * p the integer in [1, S) coprime to S closest to 0.382 S (smaller on a tie; 1 when S <= 2).  x0 = 0 (init_fbp = 0) or
+ * x0 = max(0, ipdm_fbp_forward(sino)) (init_fbp = 1, unsharpened; then the first subset is projected too); per subset
+ * r = (b - A_s x) / R (0 where R = A 1 is 0), x <- max(0, x + relaxation * A_s^T r / C_s) where C_s = A_s^T 1 > 0.  After every
+ * sweep ntv steps of normalised steepest descent on TV_eps(x) = sum sqrt(dx^2 + dy^2 + tv_eps^2) (forward differences in the
+ * native frame, 0 where they would leave the image): x <- max(0, x - t g / |g|_2), g = grad TV_eps(x), per slice,
+ * t = tv_alpha |x - x_prev|_2 with x_prev the iterate before the sweep (no change where |g| = 0); ntv = 0 with init_fbp = 0 is
+ * plain SART.  Norms are fp64 sums in a fixed order: results are bit-identical from run to run and per slice, and flip = 1 gives
+ * the column mirror of flip = 0 bit for bit.  iterations >= 1 sweeps, 0 < relaxation < 2, ntv >= 0, tv_alpha and tv_eps finite
+ * and > 0, init_fbp in {0, 1}, img must not alias sino and must be 16-byte aligned when ntv > 0 or init_fbp = 1.  R and C_s are
+ * built in the plan by the first call for a given S (that call synchronises the stream and cannot be captured); the TV scratch
+ * (2 images + 4.1 KB per slice) lives in the plan; later calls of the same or a smaller shape allocate nothing and do not
+ * synchronise. */
 int ipdm_fbp_sart_tv(ipdm_fbp_plan* plan, const float* sino_dev, float* img_dev, int batch, int flip, int iterations, int subsets,
                      float relaxation, int ntv, float tv_alpha, float tv_eps, int init_fbp, void* stream);
 /* The TV steps alone, in place on img [B,512,512] (frame flip): `steps` steps of length `step` (the same for every slice) as in
@@ -127,10 +124,11 @@ int ipdm_fbp_tv_descent(ipdm_fbp_plan* plan, float* img_dev, int batch, int flip
  * Phi(x) = 1/2 sum_i w_i ([A x]_i - b_i)^2 + beta R(x), x >= 0, A the matrix of ipdm_fbp_project, b = sino, with the weights
  * w_i = 1 / sigma^2(max(b_i, 0)), sigma^2(p) = e^p / (f N0) (1 + Ne e^p / (f N0)), f = dose, N0 = 1.4e5, Ne = 5.8 (the variance of
  * a measurement at dose f, as ipdm_low_dose_noise simulates it), computed from b in fp32, and the hyperbola penalty of
- * ipdm_fbp_pwls_penalty.  D^L = A^T (w o A 1) once per call; subsets and visit order of ipdm_fbp_sart; per subset
+ * ipdm_fbp_pwls_penalty.  D^L = A^T (w o A 1) once per call; subsets and visit order of ipdm_fbp_sart_tv; per subset
  * x <- max(0, x + (S A_s^T (w_s o (b_s - A_s x)) - beta grad R(x)) / (D^L + beta d^R(x))) (x kept where the denominator is 0).
- * x0 = 0 (init_fbp = 0) or max(0, ipdm_fbp_forward(sino)) (init_fbp = 1).  Checks of ipdm_fbp_sart (without relaxation) plus dose
- * in (0, 1], beta finite and >= 0, delta (1/cm) finite and > 0, init_fbp in {0, 1}, img 16-byte aligned.  No atomics: bit-identical
+ * x0 = 0 (init_fbp = 0) or max(0, ipdm_fbp_forward(sino)) (init_fbp = 1).  iterations, subsets and aliasing as for
+ * ipdm_fbp_sart_tv, dose in (0, 1], beta finite and >= 0, delta (1/cm) finite and > 0, init_fbp in {0, 1}, img 16-byte aligned.
+ * No atomics: bit-identical
  * from run to run and per slice, flip = 1 gives the column mirror of flip = 0.  The first call builds R = A 1 and synchronises;
  * the workspace (3 images per slice) lives in the plan; after the first call of a shape a call allocates nothing and does not
  * synchronise. */

@@ -11,9 +11,9 @@ Additive: `project(img, flip=True)` / `project_device(img)`, the forward project
 for sample.
 
 Additive: `sart(pj, flip=True, **kw)` / `sart_device(pj)`, an iterative convertor (ordered-subset SART on the projector and its
-exact adjoint, include/ipdm_b200.h ipdm_fbp_sart; with ntv > 0 or init="fbp" SART-TV, ipdm_fbp_sart_tv) with `convert`'s
-contract.  It is not the reference's ART convertor (TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector):
-its TV steps are ASD-POCS steps on a smoothed isotropic TV, not the NSL0 formula.
+exact adjoint, SART-TV with ntv > 0, include/ipdm_b200.h ipdm_fbp_sart_tv) with `convert`'s contract.  It is not the reference's
+ART convertor (TASART2DNSL0.pyd: SART with an NSL0-TV step and the area-integral projector): its TV steps are ASD-POCS steps on a
+smoothed isotropic TV, not the NSL0 formula.
 
 Additive: `pwls(pj, flip=True, **kw)` / `pwls_device(pj)`, a statistically weighted iterative convertor (penalised weighted
 least squares with dose-aware weights, solved by ordered-subset SQS, include/ipdm_b200.h ipdm_fbp_pwls) with `convert`'s contract.
@@ -47,14 +47,19 @@ class FBP:
         with torch.cuda.device(self.device):
             return self._plan.project(img.contiguous().float(), flip=flip)
 
+    def _on_host(self, device_call, a, flip, **kw):
+        """`convert`'s contract around a device call: ndarray or Tensor, one slice or a batch, in; the same kind out, float32 on
+        the host."""
+        as_tensor = isinstance(a, torch.Tensor)
+        x = a.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+        x = x[None] if x.dim() == 2 else x
+        out = device_call(x.to(self.device), flip, **kw).cpu()
+        return out if as_tensor else out.numpy()
+
     def project(self, img, flip=True):
         """`convert`'s contract in the other direction: ndarray or Tensor [B,512,512] / [512,512] in, the same kind out,
         [B,2000,912] float32 on the host."""
-        as_tensor = isinstance(img, torch.Tensor)
-        x = img.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(img, dtype=np.float32))
-        x = x[None] if x.dim() == 2 else x
-        out = self.project_device(x.to(self.device), flip).cpu()
-        return out if as_tensor else out.numpy()
+        return self._on_host(self.project_device, img, flip)
 
     def sart_device(self, pj, flip=True, **kw):
         """Iterative convertor: [B,2000,912] CUDA line integrals -> [B,512,512] CUDA image by ordered-subset SART (keywords
@@ -66,11 +71,7 @@ class FBP:
     def sart(self, pj, flip=True, **kw):
         """`convert`'s contract with SART instead of FBP: ndarray or Tensor [B,2000,912] / [2000,912] in, the same kind out,
         [B,512,512] float32 on the host."""
-        as_tensor = isinstance(pj, torch.Tensor)
-        x = pj.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(pj, dtype=np.float32))
-        x = x[None] if x.dim() == 2 else x
-        out = self.sart_device(x.to(self.device), flip, **kw).cpu()
-        return out if as_tensor else out.numpy()
+        return self._on_host(self.sart_device, pj, flip, **kw)
 
     def pwls_device(self, pj, flip=True, **kw):
         """Statistically weighted convertor: [B,2000,912] CUDA line integrals -> [B,512,512] CUDA image by PWLS / OS-SQS (keywords
@@ -81,11 +82,7 @@ class FBP:
     def pwls(self, pj, flip=True, **kw):
         """`convert`'s contract with PWLS instead of FBP: ndarray or Tensor [B,2000,912] / [2000,912] in, the same kind out,
         [B,512,512] float32 on the host."""
-        as_tensor = isinstance(pj, torch.Tensor)
-        x = pj.detach().float() if as_tensor else torch.from_numpy(np.ascontiguousarray(pj, dtype=np.float32))
-        x = x[None] if x.dim() == 2 else x
-        out = self.pwls_device(x.to(self.device), flip, **kw).cpu()
-        return out if as_tensor else out.numpy()
+        return self._on_host(self.pwls_device, pj, flip, **kw)
 
     def convert(self, pj, flip=True):
         as_tensor = isinstance(pj, torch.Tensor)

@@ -202,21 +202,30 @@ class progressive_domain_denoiser:
     def init_convertor(self, convertor):
         self._drop_graph()
         self._fbp, self._fbp_cap = None, 0
-        if convertor == "FBP":
+        if convertor in ("FBP", "SART", "PWLS"):
             self._fbp = FBP(device=self.opt.device)
-            self.convertor = self._fbp.convert
-        elif convertor == "SART":
-            self._fbp = FBP(device=self.opt.device)
-            self.convertor = lambda pj, flip=True: self._fbp.sart(pj, flip, **self._sart_kw())
-        elif convertor == "PWLS":
-            self._fbp = FBP(device=self.opt.device)
-            self.convertor = lambda pj, flip=True: self._fbp.pwls(pj, flip, **self._pwls_kw())
-        else:
-            def _unsupported(*a, **k):
-                raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP', 'SART' and 'PWLS'; the ART "
-                                   "extension TASART2DNSL0.pyd is Windows-only): call update_opt(dict(convertor='FBP'))")
-            self.convertor = _unsupported
+        def host(pj, flip=True):
+            call, _, kw = self._convertor_call(convertor)
+            return call(pj, flip, **kw)
+        self.convertor = host
         self.projection = functools.partial(proj_torch, lut_area=None, betas=None)
+
+    def _convertor_call(self, convertor, dose=None):
+        """(host call, device call, keywords) of `convertor` on the FBP plan, with the options it reads taken from opt at call time
+        (update_opt needs no re-init): FBP reads none (its host call is `convert`); SART reads the sart_* options and the TV options
+        of SART-TV (ntv, tv_alpha, tv_eps, sart_init); PWLS reads sart_iterations, sart_subsets, sart_init, pwls_beta, pwls_delta
+        and the data's dose (opt.dose unless given).  RuntimeError for any other convertor."""
+        o, f = self.opt, self._fbp
+        if convertor == "FBP":
+            return f.convert, f.convert_device, {}
+        if convertor == "SART":
+            return f.sart, f.sart_device, dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation,
+                                               ntv=o.ntv, tv_alpha=o.tv_alpha, tv_eps=o.tv_eps, init=o.sart_init)
+        if convertor == "PWLS":
+            return f.pwls, f.pwls_device, dict(iterations=o.sart_iterations, subsets=o.sart_subsets, dose=o.dose if dose is None else dose,
+                                               beta=o.pwls_beta, delta=o.pwls_delta, init=o.sart_init)
+        raise RuntimeError(f"convertor={convertor!r} is not available in the B200 build (only 'FBP', 'SART' and 'PWLS'; the ART "
+                           "extension TASART2DNSL0.pyd is Windows-only): call update_opt(dict(convertor='FBP'))")
 
     def load_model(self):
         self._drop_graph()
@@ -277,32 +286,15 @@ class progressive_domain_denoiser:
                 self._drop_graph()
             self._fbp_cap = int(batch)
 
-    def _sart_kw(self):
-        """The sart_* options and the TV options of SART-TV (ntv, tv_alpha, tv_eps, sart_init), read at call time (update_opt needs
-        no re-init)."""
-        o = self.opt
-        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, relaxation=o.sart_relaxation, ntv=o.ntv, tv_alpha=o.tv_alpha,
-                    tv_eps=o.tv_eps, init=o.sart_init)
-
-    def _pwls_kw(self, dose=None):
-        """The options convertor="PWLS" reads (sart_iterations, sart_subsets, sart_init, pwls_beta, pwls_delta and the data's dose,
-        opt.dose unless given), at call time."""
-        o = self.opt
-        return dict(iterations=o.sart_iterations, subsets=o.sart_subsets, dose=o.dose if dose is None else dose, beta=o.pwls_beta,
-                    delta=o.pwls_delta, init=o.sart_init)
-
     def _convert_device(self, sino, dose=None):
-        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan: SART when opt.convertor is 'SART', PWLS (weights at
-        `dose`, default opt.dose) when it is 'PWLS', FBP otherwise."""
+        """[B,1,2000,912] device -> [B,1,512,512] device through the FBP plan with opt.convertor (PWLS weights the rays at `dose`,
+        default opt.dose)."""
         self._reserve_fbp(sino.shape[0])
         G = 10 if self.opt.clip_proj else 1
         s = sino[:, 0].float()
         s = s * G if G != 1 else s
-        if self.opt.convertor == "SART":
-            return self._fbp.sart_device(s, **self._sart_kw())[:, None]
-        if self.opt.convertor == "PWLS":
-            return self._fbp.pwls_device(s, **self._pwls_kw(dose))[:, None]
-        return self._fbp.convert_device(s)[:, None]
+        _, call, kw = self._convertor_call(self.opt.convertor, dose)
+        return call(s, **kw)[:, None]
 
     def simulate_low_dose(self, fd, dose=None, slice_ids=None):
         """Low-dose inputs at `dose` (default opt.dose) from a full-dose batch: a sinogram [B,1,2000,912] gets the dose-reduction

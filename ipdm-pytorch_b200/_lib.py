@@ -52,7 +52,6 @@ _SIGNATURES = {
     "ipdm_fbp_tables": (ctypes.c_int, [vp, vp, vp, vp, vp]),
     "ipdm_fbp_project": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
     "ipdm_fbp_project_adjoint": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, vp]),
-    "ipdm_fbp_sart": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, vp]),
     "ipdm_fbp_sart_tv": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int,
                                         ctypes.c_float, ctypes.c_float, ctypes.c_int, vp]),
     "ipdm_fbp_tv_descent": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_float, vp]),

@@ -225,16 +225,6 @@ fbp_backproject_kernel(const float* __restrict__ q, float* __restrict__ img, con
     for (int p = 0; p < PX; ++p) ob[(size_t)(i_base + 8 * p) * NP + jo] = acc[p];
 }
 
-int ensure_workspace(ipdm_fbp_plan* plan, int batch) {
-    if (batch <= plan->cap) return IPDM_OK;
-    if (plan->d_work) IPDM_CHECK_CUDA(cudaFree(plan->d_work));
-    plan->d_work = nullptr;
-    plan->cap = 0;
-    IPDM_CHECK_CUDA(cudaMalloc(&plan->d_work, (size_t)batch * NV * ND * sizeof(float)));
-    plan->cap = batch;
-    return IPDM_OK;
-}
-
 }  // namespace ipdm
 
 using namespace ipdm;
@@ -266,15 +256,16 @@ extern "C" int ipdm_fbp_plan_create(ipdm_fbp_plan** out, int max_batch) {
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_htap, htap.data(), 2 * NTAP * sizeof(float), cudaMemcpyHostToDevice));
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_cs, cs.data(), NV * sizeof(float2), cudaMemcpyHostToDevice));
     IPDM_CHECK_CUDA(cudaMemcpy(p->d_ray, ray.data(), ND * sizeof(float2), cudaMemcpyHostToDevice));
-    if (max_batch > 0) IPDM_CHECK(ensure_workspace(p, max_batch));
+    IPDM_CHECK(p->work.reserve(work_bytes(max_batch)));
     *out = p;
     return IPDM_OK;
 }
 
 extern "C" int ipdm_fbp_plan_destroy(ipdm_fbp_plan* p) {
     if (!p) return IPDM_OK;
-    cudaFree(p->d_wcos); cudaFree(p->d_htap); cudaFree(p->d_cs); cudaFree(p->d_ray); cudaFree(p->d_work);
-    release_sart(p);
+    cudaFree(p->d_wcos); cudaFree(p->d_htap); cudaFree(p->d_cs); cudaFree(p->d_ray); cudaFree(p->d_rowsum);
+    for (auto& kv : p->colsum) cudaFree(kv.second);
+    for (GrowBuffer* b : {&p->work, &p->subset, &p->tv, &p->pwls}) b->release();
     delete p;
     return IPDM_OK;
 }
@@ -317,9 +308,9 @@ extern "C" int ipdm_fbp_backproject(ipdm_fbp_plan* p, const float* q, float* img
 
 extern "C" int ipdm_fbp_forward(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, void* stream) {
     IPDM_REQUIRE(p && sino && img && batch > 0, "ipdm_fbp_forward: bad arguments");
-    IPDM_CHECK(ensure_workspace(p, batch));
-    IPDM_CHECK(ipdm_fbp_filter(p, sino, p->d_work, batch, flip, stream));
-    return ipdm_fbp_backproject(p, p->d_work, img, batch, flip, stream);
+    IPDM_CHECK(p->work.reserve(work_bytes(batch)));
+    IPDM_CHECK(ipdm_fbp_filter(p, sino, p->work.f32(), batch, flip, stream));
+    return ipdm_fbp_backproject(p, p->work.f32(), img, batch, flip, stream);
 }
 
 extern "C" int ipdm_fbp_convert_host(ipdm_fbp_plan* p, const float* sino_host, float* img_host, int batch, int flip) {

@@ -17,6 +17,28 @@ struct FbpTables {
     double dtheta, D, da;
 };
 
+// a device buffer that grows to the largest size a call has asked of it and is never shrunk, so that after the first call of a
+// shape a call allocates nothing; it holds nothing from one call to the next
+struct GrowBuffer {
+    void* ptr = nullptr;
+    size_t bytes = 0;
+    int reserve(size_t need) {
+        if (need <= bytes) return IPDM_OK;
+        IPDM_CHECK_CUDA(cudaFree(ptr));
+        ptr = nullptr;
+        bytes = 0;
+        IPDM_CHECK_CUDA(cudaMalloc(&ptr, need));
+        bytes = need;
+        return IPDM_OK;
+    }
+    void release() {
+        cudaFree(ptr);
+        ptr = nullptr;
+        bytes = 0;
+    }
+    float* f32() const { return static_cast<float*>(ptr); }
+};
+
 }  // namespace ipdm
 
 struct ipdm_fbp_plan {
@@ -25,44 +47,29 @@ struct ipdm_fbp_plan {
     float* d_htap = nullptr;     // [2][911]  H_c[d + 455] = h[2d + 2c - 1 + 911]
     float2* d_cs = nullptr;      // [2000] (cos theta, sin theta) from fp64
     float2* d_ray = nullptr;     // [912] (cos alpha, sin alpha) from fp64, alpha = nda[k] + da/2: the fan angle filtered sample k is read at
-    float* d_work = nullptr;     // filtered sinograms [cap][2000][912]; the projector's transposed images [cap][512][512]
-    int cap = 0;
     float h0 = 0.f, inv_da = 0.f, u_off = 0.f, dtheta_f = 0.f;
     double dtheta = 0.0;
-    // SART (sart.cu): row sums R = A 1 [2000][912] (native detector order), column sums C_s = A_s^T 1 [S][512][512] (native
-    // columns) per subset count S, and the subset projections [sart_bytes / 4]; all built by the first call that needs them
+    // SART (sart.cu): row sums R = A 1 [2000][912] (native detector order) and column sums C_s = A_s^T 1 [S][512][512] (native
+    // columns) per subset count S, built by the first call that needs them and kept
     float* d_rowsum = nullptr;
     std::map<int, float*> colsum;
-    float* d_sart = nullptr;
-    size_t sart_bytes = 0;
-    // TV steps (tv.cu): g and x_prev [tv_cap][512][512] f32, per-tile partial sums [tv_cap][2][256] and step lengths [tv_cap] f64
-    void* d_tv = nullptr;
-    int tv_cap = 0;
-    // PWLS (pwls.cu): D^L, grad R and d^R [pwls_cap][512][512] f32 each
-    float* d_pwls = nullptr;
-    int pwls_cap = 0;
+    // per-call scratch, laid out for the call's batch B.  work: the filtered sinograms [B][2000][912], or the projector's transposed
+    // images [B][512][512], always reserved at the sinograms' size (work_bytes) so that only a larger batch grows it
+    ipdm::GrowBuffer work;
+    ipdm::GrowBuffer subset;     // the subset projections A_s x [B][2000 / S][912] (SART, PWLS)
+    ipdm::GrowBuffer tv;         // the TV steps (tv.cu): see tv_scratch_bytes
+    ipdm::GrowBuffer pwls;       // PWLS: D^L, grad R and d^R [B][512][512] f32 each
 };
 
 namespace ipdm {
-// grows plan->d_work to `batch` filtered sinograms (it is never shrunk)
-int ensure_workspace(ipdm_fbp_plan* plan, int batch);
-// frees the SART tables and workspace (sart.cu)
-void release_sart(ipdm_fbp_plan* plan);
-// grows the TV workspace to `batch` slices (it is never shrunk); frees it (tv.cu)
-int ensure_tv_workspace(ipdm_fbp_plan* plan, int batch);
-void release_tv(ipdm_fbp_plan* plan);
-// the workspace's x_prev images [tv_cap][512][512], the iterate before a SART sweep
-float* tv_prev(ipdm_fbp_plan* plan);
-// `steps` TV steps on img [B][512][512] (column-flipped iff flip), in place.  sweep: the step length is alpha_or_step times
-// |img - tv_prev| of each slice, taken at the first step; otherwise alpha_or_step itself (tv.cu)
+inline size_t work_bytes(int batch) { return (size_t)batch * IPDM_N_VIEWS * IPDM_N_DET * sizeof(float); }
+// the TV scratch of `batch` slices in plan->tv: x_prev (the iterate before a SART sweep, first, so at plan->tv.ptr) and g
+// [B][512][512] f32, per-tile partial sums [B][2][256] and step lengths [B] f64 (tv.cu)
+size_t tv_scratch_bytes(int batch);
+// `steps` TV steps on img [B][512][512] (column-flipped iff flip), in place, in plan->tv (reserved by the caller for `batch`).
+// sweep: the step length is alpha_or_step times |img - x_prev| of each slice, taken at the first step; otherwise alpha_or_step
+// itself (tv.cu)
 int launch_tv(ipdm_fbp_plan* p, float* img, int batch, int flip, int steps, bool sweep, double alpha_or_step, float eps, cudaStream_t st);
-// grows the PWLS workspace to `batch` slices (it is never shrunk); frees it; its D^L, grad R and d^R planes [pwls_cap][512][512]
-// (pwls.cu)
-int ensure_pwls_workspace(ipdm_fbp_plan* plan, int batch);
-void release_pwls(ipdm_fbp_plan* plan);
-float* pwls_dl(ipdm_fbp_plan* plan);
-float* pwls_grad(ipdm_fbp_plan* plan);
-float* pwls_curv(ipdm_fbp_plan* plan);
 // grad R and d^R of the hyperbola penalty of img [B][512][512] (column-flipped iff flip), in the same frame (pwls.cu)
 int launch_pwls_penalty(const float* img, float* grad, float* curv, int batch, int flip, float delta, cudaStream_t st);
 // transpose + Joseph projection of the views v0 + n * vstep, n < nv: img [B][512][512] -> sino [B][nv][912] (project.cu)

@@ -113,11 +113,12 @@ low_dose_noise_kernel(const float* sino, const float* __restrict__ noise, float*
 }
 
 int launch_project(ipdm_fbp_plan* p, const float* img, float* sino, int batch, int flip, int v0, int vstep, int nv, cudaStream_t st) {
-    IPDM_CHECK(ensure_workspace(p, batch));
-    project_transpose_kernel<<<dim3(NP / 32, NP / 32, batch), dim3(32, 8), 0, st>>>(img, p->d_work, flip);
+    IPDM_CHECK(p->work.reserve(work_bytes(batch)));
+    float* imgT = p->work.f32();
+    project_transpose_kernel<<<dim3(NP / 32, NP / 32, batch), dim3(32, 8), 0, st>>>(img, imgT, flip);
     count_launch();
     IPDM_CHECK_LAUNCH();
-    fbp_project_kernel<<<dim3(ceil_div((long long)nv * ND, PROJ_THREADS), batch), PROJ_THREADS, 0, st>>>(img, p->d_work, sino, p->d_cs,
+    fbp_project_kernel<<<dim3(ceil_div((long long)nv * ND, PROJ_THREADS), batch), PROJ_THREADS, 0, st>>>(img, imgT, sino, p->d_cs,
                                                                                                           p->d_ray, flip, v0, vstep, nv);
     count_launch();
     IPDM_CHECK_LAUNCH();

@@ -69,27 +69,6 @@ int launch_pwls_penalty(const float* img, float* grad, float* curv, int batch, i
     return IPDM_OK;
 }
 
-int ensure_pwls_workspace(ipdm_fbp_plan* p, int batch) {
-    if (batch <= p->pwls_cap) return IPDM_OK;
-    IPDM_CHECK_CUDA(cudaFree(p->d_pwls));
-    p->d_pwls = nullptr;
-    p->pwls_cap = 0;
-    IPDM_CHECK_CUDA(cudaMalloc(&p->d_pwls, (size_t)3 * batch * PW_NP * PW_NP * sizeof(float)));
-    p->pwls_cap = batch;
-    return IPDM_OK;
-}
-
-void release_pwls(ipdm_fbp_plan* p) {
-    cudaFree(p->d_pwls);
-    p->d_pwls = nullptr;
-    p->pwls_cap = 0;
-}
-
-// workspace of capacity cap: D^L, grad R, d^R, each [cap][512][512] f32
-float* pwls_dl(ipdm_fbp_plan* p) { return p->d_pwls; }
-float* pwls_grad(ipdm_fbp_plan* p) { return p->d_pwls + (size_t)p->pwls_cap * PW_NP * PW_NP; }
-float* pwls_curv(ipdm_fbp_plan* p) { return p->d_pwls + (size_t)2 * p->pwls_cap * PW_NP * PW_NP; }
-
 }  // namespace ipdm
 
 using namespace ipdm;

@@ -20,7 +20,7 @@
 //           w(b) = 1 / sigma^2(max(b, 0)) computed from b in fp32 (no weight sinogram is stored).
 // Kernel 2  fill_kernel                the all-ones image / sinogram the tables R = A 1 and C_s = A_s^T 1 are computed from.
 // Kernel 3  clamp_nonneg_kernel        x0 = max(0, FBP) of the FBP start.
-// SART-TV: before every sweep the iterate is copied to the TV workspace's x_prev, after it ntv TV steps run (launch_tv).
+// SART-TV: before every sweep the iterate is copied to x_prev in the TV scratch, after it ntv TV steps run (launch_tv).
 // PWLS: D^L once per call, then per subset transpose, projection, penalty (launch_pwls_penalty) and the SQS adjoint.
 #include "fbp_plan.cuh"
 
@@ -261,10 +261,10 @@ static int ensure_rowsum(ipdm_fbp_plan* p, const char* fn, cudaStream_t st) {
 
 // R (ensure_rowsum) and C_s = A_s^T 1 for every subset of S (once per plan and S), in fp32 with the same kernels
 static int ensure_sart_tables(ipdm_fbp_plan* p, int S, cudaStream_t st) {
-    IPDM_CHECK(ensure_rowsum(p, "ipdm_fbp_sart", st));
+    IPDM_CHECK(ensure_rowsum(p, "ipdm_fbp_sart_tv", st));
     if (p->colsum.count(S)) return IPDM_OK;
     char what[96];
-    snprintf(what, sizeof what, "ipdm_fbp_sart: the first call with %d subsets builds the plan's tables and", S);
+    snprintf(what, sizeof what, "ipdm_fbp_sart_tv: the first call with %d subsets builds the plan's tables and", S);
     IPDM_CHECK(require_eager(st, what));
     float* ones = nullptr;
     IPDM_CHECK(make_ones(&ones, st));
@@ -274,31 +274,7 @@ static int ensure_sart_tables(ipdm_fbp_plan* p, int S, cudaStream_t st) {
         rc = launch_adjoint<ADJ_PLAIN>(p, ones, nullptr, nullptr, c + (size_t)s * NP * NP, 1, 0, s, S, NV / S, 0.f, st);
     if (rc == IPDM_OK) p->colsum[S] = c;
     else cudaFree(c);
-    return finish_build(rc, ones, "ipdm_fbp_sart", st);
-}
-
-void release_sart(ipdm_fbp_plan* p) {
-    cudaFree(p->d_rowsum);
-    cudaFree(p->d_sart);
-    for (auto& kv : p->colsum) cudaFree(kv.second);
-    p->d_rowsum = p->d_sart = nullptr;
-    p->colsum.clear();
-    p->sart_bytes = 0;
-    release_tv(p);
-    release_pwls(p);
-}
-
-// grows the subset projections A_s x to `batch` slices of nv views (never shrunk)
-static int ensure_subset_buffer(ipdm_fbp_plan* p, int batch, int nv) {
-    const size_t need = (size_t)batch * nv * ND * sizeof(float);
-    if (need > p->sart_bytes) {
-        IPDM_CHECK_CUDA(cudaFree(p->d_sart));
-        p->d_sart = nullptr;
-        p->sart_bytes = 0;
-        IPDM_CHECK_CUDA(cudaMalloc(&p->d_sart, need));
-        p->sart_bytes = need;
-    }
-    return IPDM_OK;
+    return finish_build(rc, ones, "ipdm_fbp_sart_tv", st);
 }
 
 // the start of an iterative convertor: x0 = max(0, FBP(sino)), unsharpened (init_fbp = 1), or x0 = 0
@@ -315,27 +291,34 @@ static int set_start(ipdm_fbp_plan* p, const float* sino, float* img, int batch,
     return IPDM_OK;
 }
 
-// SART (ntv = 0) or SART-TV, from x0 = 0 (init_fbp = 0) or x0 = max(0, FBP(sino)) (init_fbp = 1); arguments checked by the callers
+// proj = A_s x of the iterate, in the plan's subset buffer (reserved by the caller), or null when x is known to be 0: A_s 0 = 0,
+// so the first subset from the zero start needs no projection
+static int project_subset(ipdm_fbp_plan* p, const float* img, bool zero, int batch, int flip, int s, int subsets, const float** proj,
+                          cudaStream_t st) {
+    *proj = nullptr;
+    if (zero) return IPDM_OK;
+    *proj = p->subset.f32();
+    return launch_project(p, img, p->subset.f32(), batch, flip, s, subsets, NV / subsets, st);
+}
+
+// SART (ntv = 0) or SART-TV, from x0 = 0 (init_fbp = 0) or x0 = max(0, FBP(sino)) (init_fbp = 1); arguments checked by the caller
 static int run_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets, float relaxation,
                     int ntv, float tv_alpha, float tv_eps, int init_fbp, cudaStream_t st) {
     IPDM_CHECK(ensure_sart_tables(p, subsets, st));
-    IPDM_CHECK(ensure_workspace(p, batch));                                    // the projector's transposed iterates
-    if (ntv > 0) IPDM_CHECK(ensure_tv_workspace(p, batch));                    // g, x_prev and the partial sums of the TV steps
     const int nv = NV / subsets;
-    IPDM_CHECK(ensure_subset_buffer(p, batch, nv));                            // A_s x of one subset
+    IPDM_CHECK(p->work.reserve(work_bytes(batch)));                           // the projector's transposed iterates
+    IPDM_CHECK(p->subset.reserve((size_t)batch * nv * ND * sizeof(float)));   // A_s x of one subset
+    if (ntv > 0) IPDM_CHECK(p->tv.reserve(tv_scratch_bytes(batch)));           // x_prev, g and the partial sums of the TV steps
     const float* colsum = p->colsum[subsets];
     const int step = sart_visit_step(subsets);
     const size_t img_bytes = (size_t)batch * NP * NP * sizeof(float);
     IPDM_CHECK(set_start(p, sino, img, batch, flip, init_fbp, st));
     for (int it = 0; it < iterations; ++it) {
-        if (ntv > 0) IPDM_CHECK_CUDA(cudaMemcpyAsync(tv_prev(p), img, img_bytes, cudaMemcpyDeviceToDevice, st));
+        if (ntv > 0) IPDM_CHECK_CUDA(cudaMemcpyAsync(p->tv.ptr, img, img_bytes, cudaMemcpyDeviceToDevice, st));     // x_prev
         for (int n = 0; n < subsets; ++n) {
             const int s = (int)((long long)n * step % subsets);
-            const float* proj = nullptr;                                       // A_s x0 = 0: the first subset from 0 needs no projection
-            if (init_fbp || it > 0 || n > 0) {
-                IPDM_CHECK(launch_project(p, img, p->d_sart, batch, flip, s, subsets, nv, st));
-                proj = p->d_sart;
-            }
+            const float* proj;
+            IPDM_CHECK(project_subset(p, img, !init_fbp && it == 0 && n == 0, batch, flip, s, subsets, &proj, st));
             IPDM_CHECK(launch_adjoint<ADJ_SART>(p, sino, proj, colsum + (size_t)s * NP * NP, img, batch, flip, s, subsets, nv, relaxation,
                                                 st));
         }
@@ -348,28 +331,29 @@ static int run_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, 
 static int run_pwls(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets, float dose,
                     float beta, float delta, int init_fbp, cudaStream_t st) {
     IPDM_CHECK(ensure_rowsum(p, "ipdm_fbp_pwls", st));                         // R, no C_s tables
-    IPDM_CHECK(ensure_workspace(p, batch));
-    IPDM_CHECK(ensure_pwls_workspace(p, batch));                               // D^L, grad R, d^R
     const int nv = NV / subsets;
-    IPDM_CHECK(ensure_subset_buffer(p, batch, nv));
+    const size_t plane = (size_t)batch * NP * NP;
+    IPDM_CHECK(p->work.reserve(work_bytes(batch)));
+    IPDM_CHECK(p->subset.reserve((size_t)batch * nv * ND * sizeof(float)));
+    IPDM_CHECK(p->pwls.reserve(3 * plane * sizeof(float)));
+    float* dl = p->pwls.f32();
+    float* grad = dl + plane;
+    float* curv = grad + plane;
     PwlsArgs pw;
-    pw.dl = pwls_dl(p);
-    pw.grad = pwls_grad(p);
-    pw.curv = pwls_curv(p);
+    pw.dl = dl;
+    pw.grad = grad;
+    pw.curv = curv;
     pw.wk = (float)(1.0 / ((double)dose * kDoseN0));
     pw.beta = beta;
-    IPDM_CHECK(launch_adjoint<ADJ_DENOM>(p, sino, nullptr, nullptr, pwls_dl(p), batch, flip, 0, 1, NV, 0.f, st, pw));
+    IPDM_CHECK(launch_adjoint<ADJ_DENOM>(p, sino, nullptr, nullptr, dl, batch, flip, 0, 1, NV, 0.f, st, pw));
     IPDM_CHECK(set_start(p, sino, img, batch, flip, init_fbp, st));
     const int step = sart_visit_step(subsets);
     for (int it = 0; it < iterations; ++it) {
         for (int n = 0; n < subsets; ++n) {
             const int s = (int)((long long)n * step % subsets);
-            const float* proj = nullptr;                                       // A_s x0 = 0: the first subset from 0 needs no projection
-            if (init_fbp || it > 0 || n > 0) {
-                IPDM_CHECK(launch_project(p, img, p->d_sart, batch, flip, s, subsets, nv, st));
-                proj = p->d_sart;
-            }
-            IPDM_CHECK(launch_pwls_penalty(img, pwls_grad(p), pwls_curv(p), batch, flip, delta, st));
+            const float* proj;
+            IPDM_CHECK(project_subset(p, img, !init_fbp && it == 0 && n == 0, batch, flip, s, subsets, &proj, st));
+            IPDM_CHECK(launch_pwls_penalty(img, grad, curv, batch, flip, delta, st));
             IPDM_CHECK(launch_adjoint<ADJ_SQS>(p, sino, proj, nullptr, img, batch, flip, s, subsets, nv, (float)subsets, st, pw));
         }
     }
@@ -385,29 +369,23 @@ extern "C" int ipdm_fbp_project_adjoint(ipdm_fbp_plan* p, const float* sino, flo
     return launch_adjoint<ADJ_PLAIN>(p, sino, nullptr, nullptr, img, batch, flip, 0, 1, NV, 0.f, (cudaStream_t)stream);
 }
 
-// the argument checks all iterative entries share, and the relaxation of the SART entries
+// the argument checks both iterative entries share
 #define ITER_CHECK_ARGS(fn)                                                                                                       \
     IPDM_REQUIRE(p && sino && img && sino != img && batch > 0 && batch <= 65535, fn ": bad arguments");                          \
     IPDM_REQUIRE(iterations >= 1, fn ": iterations must be >= 1, got %d", iterations);                                          \
     IPDM_REQUIRE(subsets >= 1 && subsets <= NV && NV % subsets == 0, fn ": subsets must divide %d, got %d", NV, subsets)
-#define SART_CHECK_ARGS(fn)                                                                                                       \
-    ITER_CHECK_ARGS(fn);                                                                                                          \
-    IPDM_REQUIRE(relaxation > 0.f && relaxation < 2.f, fn ": relaxation must be in (0, 2), got %g", (double)relaxation)
-
-extern "C" int ipdm_fbp_sart(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
-                             float relaxation, void* stream) {
-    SART_CHECK_ARGS("ipdm_fbp_sart");
-    return run_sart(p, sino, img, batch, flip, iterations, subsets, relaxation, 0, 0.f, 0.f, 0, (cudaStream_t)stream);
-}
 
 extern "C" int ipdm_fbp_sart_tv(ipdm_fbp_plan* p, const float* sino, float* img, int batch, int flip, int iterations, int subsets,
                                 float relaxation, int ntv, float tv_alpha, float tv_eps, int init_fbp, void* stream) {
-    SART_CHECK_ARGS("ipdm_fbp_sart_tv");
+    ITER_CHECK_ARGS("ipdm_fbp_sart_tv");
+    IPDM_REQUIRE(relaxation > 0.f && relaxation < 2.f, "ipdm_fbp_sart_tv: relaxation must be in (0, 2), got %g", (double)relaxation);
     IPDM_REQUIRE(ntv >= 0, "ipdm_fbp_sart_tv: ntv must be >= 0, got %d", ntv);
     IPDM_REQUIRE(std::isfinite(tv_alpha) && tv_alpha > 0.f, "ipdm_fbp_sart_tv: tv_alpha must be finite and > 0, got %g", (double)tv_alpha);
     IPDM_REQUIRE(std::isfinite(tv_eps) && tv_eps > 0.f, "ipdm_fbp_sart_tv: tv_eps must be finite and > 0, got %g", (double)tv_eps);
     IPDM_REQUIRE(init_fbp == 0 || init_fbp == 1, "ipdm_fbp_sart_tv: init_fbp must be 0 or 1, got %d", init_fbp);
-    IPDM_REQUIRE(((uintptr_t)img & 15) == 0, "ipdm_fbp_sart_tv: img must be 16-byte aligned");
+    // the TV steps and the FBP start's clamp work on float4
+    IPDM_REQUIRE((ntv == 0 && init_fbp == 0) || ((uintptr_t)img & 15) == 0,
+                 "ipdm_fbp_sart_tv: img must be 16-byte aligned when ntv > 0 or init_fbp = 1");
     return run_sart(p, sino, img, batch, flip, iterations, subsets, relaxation, ntv, tv_alpha, tv_eps, init_fbp, (cudaStream_t)stream);
 }
 

@@ -137,40 +137,25 @@ tv_update_kernel(float* __restrict__ x, const float* __restrict__ g, const doubl
     }
 }
 
-static size_t tv_slice_bytes() { return 2 * (size_t)TV_NP * TV_NP * sizeof(float) + (2 * TV_TILES + 1) * sizeof(double); }
-
-int ensure_tv_workspace(ipdm_fbp_plan* p, int batch) {
-    if (batch <= p->tv_cap) return IPDM_OK;
-    IPDM_CHECK_CUDA(cudaFree(p->d_tv));
-    p->d_tv = nullptr;
-    p->tv_cap = 0;
-    IPDM_CHECK_CUDA(cudaMalloc(&p->d_tv, (size_t)batch * tv_slice_bytes()));
-    p->tv_cap = batch;
-    return IPDM_OK;
+size_t tv_scratch_bytes(int batch) {
+    return (size_t)batch * (2 * (size_t)TV_NP * TV_NP * sizeof(float) + (2 * TV_TILES + 1) * sizeof(double));
 }
-
-void release_tv(ipdm_fbp_plan* p) {
-    cudaFree(p->d_tv);
-    p->d_tv = nullptr;
-    p->tv_cap = 0;
-}
-
-// workspace of capacity cap: g [cap][512][512] f32, x_prev [cap][512][512] f32, partials [cap][2][256] f64, t [cap] f64
-static float* tv_g(ipdm_fbp_plan* p) { return reinterpret_cast<float*>(p->d_tv); }
-float* tv_prev(ipdm_fbp_plan* p) { return tv_g(p) + (size_t)p->tv_cap * TV_NP * TV_NP; }
-static double* tv_part(ipdm_fbp_plan* p) { return reinterpret_cast<double*>(tv_prev(p) + (size_t)p->tv_cap * TV_NP * TV_NP); }
-static double* tv_t(ipdm_fbp_plan* p) { return tv_part(p) + (size_t)p->tv_cap * 2 * TV_TILES; }
 
 int launch_tv(ipdm_fbp_plan* p, float* img, int batch, int flip, int steps, bool sweep, double alpha_or_step, float eps,
               cudaStream_t st) {
+    const size_t plane = (size_t)batch * TV_NP * TV_NP;
+    const float* xprev = p->tv.f32();
+    float* g = p->tv.f32() + plane;
+    double* part = reinterpret_cast<double*>(g + plane);
+    double* tval = part + (size_t)batch * 2 * TV_TILES;
     const dim3 gg(TV_NP / TV_T, TV_NP / TV_T, batch), gu(TV_NP * TV_NP / TV_UPD_PIX, batch);
     const float eps2 = eps * eps;
     for (int s = 0; s < steps; ++s) {
         if (sweep && s == 0)
-            tv_grad_kernel<true><<<gg, 256, 0, st>>>(img, tv_prev(p), tv_g(p), tv_part(p), eps2, flip);
+            tv_grad_kernel<true><<<gg, 256, 0, st>>>(img, xprev, g, part, eps2, flip);
         else
-            tv_grad_kernel<false><<<gg, 256, 0, st>>>(img, nullptr, tv_g(p), tv_part(p), eps2, flip);
-        tv_update_kernel<<<gu, 256, 0, st>>>(img, tv_g(p), tv_part(p), tv_t(p), sweep ? (s == 0 ? 1 : 2) : 0, alpha_or_step);
+            tv_grad_kernel<false><<<gg, 256, 0, st>>>(img, nullptr, g, part, eps2, flip);
+        tv_update_kernel<<<gu, 256, 0, st>>>(img, g, part, tval, sweep ? (s == 0 ? 1 : 2) : 0, alpha_or_step);
         count_launch(2);
         IPDM_CHECK_LAUNCH();
     }
@@ -188,6 +173,6 @@ extern "C" int ipdm_fbp_tv_descent(ipdm_fbp_plan* p, float* img, int batch, int 
     IPDM_REQUIRE(std::isfinite(eps) && eps > 0.f, "ipdm_fbp_tv_descent: eps must be finite and > 0, got %g", (double)eps);
     IPDM_REQUIRE(((uintptr_t)img & 15) == 0, "ipdm_fbp_tv_descent: img must be 16-byte aligned");
     if (steps == 0) return IPDM_OK;
-    IPDM_CHECK(ensure_tv_workspace(p, batch));
+    IPDM_CHECK(p->tv.reserve(tv_scratch_bytes(batch)));
     return launch_tv(p, img, batch, flip, steps, false, (double)step, eps, (cudaStream_t)stream);
 }

@@ -20,6 +20,7 @@ SART_TV_DEFAULTS = dict(ntv=0, tv_alpha=0.2, tv_eps=1e-4, init="zero")
 SART_INITS = ("zero", "fbp")
 # the pwls_* options of convertor="PWLS" (pwls_beta, pwls_delta in 1/cm of Config/default_config.py; DESIGN 8 has the study)
 PWLS_DEFAULTS = dict(beta=1e6, delta=0.0002)
+PWLS_DOSE = 0.25             # the dose `FBPPlan.pwls` weights the rays for when none is given (the default of the dose option)
 PRECISIONS = {"tf32": 0, "bf16": 1, "fp32": 2}
 
 
@@ -40,6 +41,25 @@ def _opt(t, name="tensor"):
 
 def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+def _real(v, name, rule, ok):
+    """float(v); ValueError "<name> must be <rule>" unless v is a finite real number (a bool or a str is not) with ok(v)."""
+    if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or not (math.isfinite(v) and ok(v)):
+        raise ValueError(f"{name} must be {rule}, got {v!r}")
+    return float(v)
+
+
+def _sweeps(who, iterations, subsets, init):
+    """(int, int, str): the sweeps, subsets and start every iterative convertor takes; ValueError unless iterations >= 1, subsets
+    divides 2000 and init is "zero" or "fbp"."""
+    if isinstance(iterations, bool) or int(iterations) != iterations or iterations < 1:
+        raise ValueError(f"{who} iterations must be an integer >= 1, got {iterations!r}")
+    if isinstance(subsets, bool) or int(subsets) != subsets or not 1 <= subsets <= N_VIEWS or N_VIEWS % int(subsets):
+        raise ValueError(f"{who} subsets must be an integer dividing {N_VIEWS}, got {subsets!r}")
+    if init not in SART_INITS:
+        raise ValueError(f"{who} init must be one of {SART_INITS}, got {init!r}")
+    return int(iterations), int(subsets), str(init)
 
 
 def launch_count():
@@ -140,104 +160,83 @@ class FBPPlan:
         check(_lib.lib().ipdm_fbp_project(self._h, _dev(img, "img"), _dev(out, "out"), b, int(bool(flip)), _stream()), "ipdm_fbp_project")
         return out
 
-    def _image_out(self, out, b, like):
-        out = torch.empty(b, N_PIX, N_PIX, device=like.device, dtype=torch.float32) if out is None else out
+    def _image_out(self, sino, out):
+        """out, or a new [B,512,512] device image, for the sinogram sino [B,2000,912]; ValueError unless both have these shapes and
+        out is not sino."""
+        self._check_sino(sino)
+        b = sino.shape[0]
+        out = torch.empty(b, N_PIX, N_PIX, device=sino.device, dtype=torch.float32) if out is None else out
         if tuple(out.shape) != (b, N_PIX, N_PIX):
             raise ValueError(f"out must be [{b},{N_PIX},{N_PIX}], got {tuple(out.shape)}")
+        if out.data_ptr() == sino.data_ptr():
+            raise ValueError("out must not alias sino")
         return out
 
     def project_adjoint(self, sino, flip=True, out=None):
         """Exact adjoint (transpose) of `project`: [B,2000,912] device -> [B,512,512] device, the same weights and flip frames, so
         <project(x), y> = <x, project_adjoint(y)> up to fp32 rounding.  Deterministic and slice by slice."""
-        self._check_sino(sino)
-        b = sino.shape[0]
-        out = self._image_out(out, b, sino)
-        check(_lib.lib().ipdm_fbp_project_adjoint(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), _stream()),
-              "ipdm_fbp_project_adjoint")
+        out = self._image_out(sino, out)
+        check(_lib.lib().ipdm_fbp_project_adjoint(self._h, _dev(sino, "sino"), _dev(out, "out"), sino.shape[0], int(bool(flip)),
+                                                  _stream()), "ipdm_fbp_project_adjoint")
         return out
+
+    @staticmethod
+    def check_sart_args(iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], relaxation=SART_DEFAULTS["relaxation"],
+                        ntv=SART_TV_DEFAULTS["ntv"], tv_alpha=SART_TV_DEFAULTS["tv_alpha"], tv_eps=SART_TV_DEFAULTS["tv_eps"],
+                        init=SART_TV_DEFAULTS["init"]):
+        """ValueError unless iterations >= 1, subsets divides 2000, 0 < relaxation < 2, ntv is an integer >= 0, tv_alpha and tv_eps
+        are finite and > 0 and init is "zero" or "fbp"; returns them as (int, int, float, int, float, float, str)."""
+        iterations, subsets, init = _sweeps("SART", iterations, subsets, init)
+        relaxation = _real(relaxation, "SART relaxation", "in (0, 2)", lambda v: 0 < v < 2)
+        if isinstance(ntv, bool) or not isinstance(ntv, (int, np.integer)) or ntv < 0:
+            raise ValueError(f"SART-TV ntv must be an integer >= 0, got {ntv!r}")
+        tv_alpha = _real(tv_alpha, "SART-TV tv_alpha", "finite and > 0", lambda v: v > 0)
+        tv_eps = _real(tv_eps, "SART-TV tv_eps", "finite and > 0", lambda v: v > 0)
+        return iterations, subsets, relaxation, int(ntv), tv_alpha, tv_eps, init
 
     @staticmethod
     def check_tv_args(ntv=SART_TV_DEFAULTS["ntv"], tv_alpha=SART_TV_DEFAULTS["tv_alpha"], tv_eps=SART_TV_DEFAULTS["tv_eps"],
                       init=SART_TV_DEFAULTS["init"]):
-        """ValueError unless ntv is an integer >= 0, tv_alpha and tv_eps are finite and > 0 and init is "zero" or "fbp"; returns
-        them as (int, float, float, str)."""
-        if isinstance(ntv, bool) or not isinstance(ntv, (int, np.integer)) or ntv < 0:
-            raise ValueError(f"SART-TV ntv must be an integer >= 0, got {ntv!r}")
-        for name, v in (("tv_alpha", tv_alpha), ("tv_eps", tv_eps)):
-            if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or not (math.isfinite(v) and v > 0):
-                raise ValueError(f"SART-TV {name} must be finite and > 0, got {v!r}")
-        if init not in SART_INITS:
-            raise ValueError(f"SART init must be one of {SART_INITS}, got {init!r}")
-        return int(ntv), float(tv_alpha), float(tv_eps), str(init)
-
-    @staticmethod
-    def check_sart_args(iterations, subsets, relaxation, **tv):
-        """ValueError unless iterations >= 1, subsets divides 2000 and 0 < relaxation < 2 (and the keywords of `check_tv_args`, when
-        given, pass it); returns (iterations, subsets, relaxation) as (int, int, float)."""
-        if isinstance(iterations, bool) or int(iterations) != iterations or iterations < 1:
-            raise ValueError(f"SART iterations must be an integer >= 1, got {iterations!r}")
-        if isinstance(subsets, bool) or int(subsets) != subsets or not 1 <= subsets <= N_VIEWS or N_VIEWS % int(subsets):
-            raise ValueError(f"SART subsets must be an integer dividing {N_VIEWS}, got {subsets!r}")
-        if not 0.0 < float(relaxation) < 2.0:
-            raise ValueError(f"SART relaxation must be in (0, 2), got {relaxation!r}")
-        FBPPlan.check_tv_args(**tv)
-        return int(iterations), int(subsets), float(relaxation)
+        """The SART-TV part of `check_sart_args`: (ntv, tv_alpha, tv_eps, init) as (int, float, float, str)."""
+        return FBPPlan.check_sart_args(ntv=ntv, tv_alpha=tv_alpha, tv_eps=tv_eps, init=init)[3:]
 
     def sart(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"],
              relaxation=SART_DEFAULTS["relaxation"], out=None, ntv=SART_TV_DEFAULTS["ntv"], tv_alpha=SART_TV_DEFAULTS["tv_alpha"],
              tv_eps=SART_TV_DEFAULTS["tv_eps"], init=SART_TV_DEFAULTS["init"]):
-        """Ordered-subset SART (see include/ipdm_b200.h ipdm_fbp_sart): line integrals [B,2000,912] device -> mu image [B,512,512]
-        device in the frame of `forward` for the same flip.  With ntv > 0 or init="fbp" it is SART-TV (ipdm_fbp_sart_tv): the
-        start is max(0, forward(sino)) for init="fbp", and every sweep is followed by ntv TV steps of length tv_alpha |x - x_prev|
-        (tv_eps in 1/cm smooths the TV).  The first call for a subset count builds the plan's tables and synchronises; later calls
-        allocate nothing (CUDA-graph safe)."""
-        self._check_sino(sino)
-        iterations, subsets, relaxation = self.check_sart_args(iterations, subsets, relaxation)
-        ntv, tv_alpha, tv_eps, init = self.check_tv_args(ntv, tv_alpha, tv_eps, init)
-        b = sino.shape[0]
-        out = self._image_out(out, b, sino)
-        if out.data_ptr() == sino.data_ptr():
-            raise ValueError("out must not alias sino")
-        if ntv == 0 and init == "zero":
-            check(_lib.lib().ipdm_fbp_sart(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
-                                           ctypes.c_float(relaxation), _stream()), "ipdm_fbp_sart")
-        else:
-            check(_lib.lib().ipdm_fbp_sart_tv(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
-                                              ctypes.c_float(relaxation), ntv, ctypes.c_float(tv_alpha), ctypes.c_float(tv_eps),
-                                              int(init == "fbp"), _stream()), "ipdm_fbp_sart_tv")
+        """Ordered-subset SART, regularised to SART-TV by ntv > 0 (see include/ipdm_b200.h ipdm_fbp_sart_tv): line integrals
+        [B,2000,912] device -> mu image [B,512,512] device in the frame of `forward` for the same flip.  The start is 0, or
+        max(0, forward(sino)) for init="fbp"; every sweep is followed by ntv TV steps of length tv_alpha |x - x_prev| (tv_eps in 1/cm
+        smooths the TV).  The first call for a subset count builds the plan's tables and synchronises; later calls allocate nothing
+        (CUDA-graph safe)."""
+        iterations, subsets, relaxation, ntv, tv_alpha, tv_eps, init = self.check_sart_args(iterations, subsets, relaxation, ntv,
+                                                                                            tv_alpha, tv_eps, init)
+        out = self._image_out(sino, out)
+        check(_lib.lib().ipdm_fbp_sart_tv(self._h, _dev(sino, "sino"), _dev(out, "out"), sino.shape[0], int(bool(flip)), iterations,
+                                          subsets, ctypes.c_float(relaxation), ntv, ctypes.c_float(tv_alpha), ctypes.c_float(tv_eps),
+                                          int(init == "fbp"), _stream()), "ipdm_fbp_sart_tv")
         return out
 
     @staticmethod
-    def check_pwls_args(iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=0.25, beta=PWLS_DEFAULTS["beta"],
-                        delta=PWLS_DEFAULTS["delta"], init=SART_TV_DEFAULTS["init"]):
+    def check_pwls_args(iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=PWLS_DOSE,
+                        beta=PWLS_DEFAULTS["beta"], delta=PWLS_DEFAULTS["delta"], init=SART_TV_DEFAULTS["init"]):
         """ValueError unless iterations >= 1, subsets divides 2000, 0 < dose <= 1, beta is finite and >= 0, delta is finite and > 0
         and init is "zero" or "fbp"; returns them as (int, int, float, float, float, str)."""
-        iterations, subsets, _ = FBPPlan.check_sart_args(iterations, subsets, 1.0)
-        real = lambda v: not isinstance(v, bool) and isinstance(v, (int, float, np.integer, np.floating)) and math.isfinite(v)
-        if not (real(dose) and 0.0 < dose <= 1.0):
-            raise ValueError(f"PWLS dose must be in (0, 1], got {dose!r}")
-        if not (real(beta) and beta >= 0):
-            raise ValueError(f"PWLS beta must be finite and >= 0, got {beta!r}")
-        if not (real(delta) and delta > 0):
-            raise ValueError(f"PWLS delta must be finite and > 0, got {delta!r}")
-        if init not in SART_INITS:
-            raise ValueError(f"PWLS init must be one of {SART_INITS}, got {init!r}")
-        return iterations, subsets, float(dose), float(beta), float(delta), str(init)
+        iterations, subsets, init = _sweeps("PWLS", iterations, subsets, init)
+        dose = _real(dose, "PWLS dose", "in (0, 1]", lambda v: 0 < v <= 1)
+        beta = _real(beta, "PWLS beta", "finite and >= 0", lambda v: v >= 0)
+        delta = _real(delta, "PWLS delta", "finite and > 0", lambda v: v > 0)
+        return iterations, subsets, dose, beta, delta, init
 
-    def pwls(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=0.25,
+    def pwls(self, sino, flip=True, iterations=SART_DEFAULTS["iterations"], subsets=SART_DEFAULTS["subsets"], dose=PWLS_DOSE,
              beta=PWLS_DEFAULTS["beta"], delta=PWLS_DEFAULTS["delta"], init=SART_TV_DEFAULTS["init"], out=None):
         """Penalised weighted least squares by ordered-subset SQS (see include/ipdm_b200.h ipdm_fbp_pwls): line integrals
         [B,2000,912] device at dose `dose` -> mu image [B,512,512] device in the frame of `forward` for the same flip.  The weights
         are the inverse variances of the rays at that dose; beta scales the hyperbola penalty, delta (1/cm) is its edge scale;
         subsets and sweeps as in `sart`; init="fbp" starts from max(0, forward(sino)).  The first call builds the plan's row sums and
         synchronises; later calls allocate nothing (CUDA-graph safe)."""
-        self._check_sino(sino)
         iterations, subsets, dose, beta, delta, init = self.check_pwls_args(iterations, subsets, dose, beta, delta, init)
-        b = sino.shape[0]
-        out = self._image_out(out, b, sino)
-        if out.data_ptr() == sino.data_ptr():
-            raise ValueError("out must not alias sino")
-        check(_lib.lib().ipdm_fbp_pwls(self._h, _dev(sino, "sino"), _dev(out, "out"), b, int(bool(flip)), iterations, subsets,
+        out = self._image_out(sino, out)
+        check(_lib.lib().ipdm_fbp_pwls(self._h, _dev(sino, "sino"), _dev(out, "out"), sino.shape[0], int(bool(flip)), iterations, subsets,
                                        ctypes.c_float(dose), ctypes.c_float(beta), ctypes.c_float(delta), int(init == "fbp"), _stream()),
               "ipdm_fbp_pwls")
         return out
@@ -247,8 +246,7 @@ class FBPPlan:
         regulariser of `pwls` on its own (include/ipdm_b200.h ipdm_fbp_pwls_penalty)."""
         if img.dim() != 3 or tuple(img.shape[1:]) != (N_PIX, N_PIX):
             raise ValueError(f"image must be [B,{N_PIX},{N_PIX}], got {tuple(img.shape)}")
-        if not (math.isfinite(delta) and delta > 0):
-            raise ValueError(f"PWLS delta must be finite and > 0, got {delta!r}")
+        delta = _real(delta, "PWLS delta", "finite and > 0", lambda v: v > 0)
         grad, curv = torch.empty_like(img), torch.empty_like(img)
         check(_lib.lib().ipdm_fbp_pwls_penalty(self._h, _dev(img, "img"), _dev(grad, "grad"), _dev(curv, "curv"), img.shape[0],
                                                int(bool(flip)), ctypes.c_float(delta), _stream()), "ipdm_fbp_pwls_penalty")
@@ -261,10 +259,8 @@ class FBPPlan:
             raise ValueError(f"image must be [B,{N_PIX},{N_PIX}], got {tuple(img.shape)}")
         if isinstance(steps, bool) or int(steps) != steps or steps < 0:
             raise ValueError(f"TV steps must be an integer >= 0, got {steps!r}")
-        if not (math.isfinite(step) and step >= 0):
-            raise ValueError(f"TV step must be finite and >= 0, got {step!r}")
-        if not (math.isfinite(eps) and eps > 0):
-            raise ValueError(f"TV eps must be finite and > 0, got {eps!r}")
+        step = _real(step, "TV step", "finite and >= 0", lambda v: v >= 0)
+        eps = _real(eps, "TV eps", "finite and > 0", lambda v: v > 0)
         check(_lib.lib().ipdm_fbp_tv_descent(self._h, _dev(img, "img"), img.shape[0], int(bool(flip)), int(steps), ctypes.c_float(step),
                                              ctypes.c_float(eps), _stream()), "ipdm_fbp_tv_descent")
         return img

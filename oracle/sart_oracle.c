@@ -1,6 +1,6 @@
 /*
  * TEST INFRASTRUCTURE ONLY -- fp64 restatement of the adjoint projector and of ordered-subset SART
- * (ipdm_fbp_project_adjoint, ipdm_fbp_sart, csrc/sart.cu).
+ * (ipdm_fbp_project_adjoint, ipdm_fbp_sart_tv with ntv = 0, csrc/sart.cu).
  *
  * The rays and Joseph weights are those of oracle/project_oracle.c (ray_sum): along the dominant axis one
  * sample per column / row m at u(m) = u0 + (m - 255.5) g, weight 1 - w on pixel floor(u) and w on floor(u) + 1
@@ -8,7 +8,7 @@
  *
  * adjoint_oracle scatters each ray's weights times its value.  Under OpenMP the views are split statically over
  * per-thread image buffers that are summed in thread order, so the result is fixed for a given thread count.
- * sart_oracle runs the loop of ipdm_fbp_sart in fp64 with R = A 1 and C_s = A_s^T 1 from the same weights.
+ * sart_oracle runs the plain SART loop of ipdm_fbp_sart_tv in fp64 with R = A 1 and C_s = A_s^T 1 from the same weights.
  * Both work in the native frame; flip = 1 reverses the detector axis of the sinogram and the columns of the image.
  * Nothing under ipdm-pytorch_b200/ links or loads this file.
  */
@@ -153,7 +153,7 @@ void adjoint_oracle(const double *sino, double *img, int batch, int nv, int flip
 
 static int gcd(int a, int b) { while (b) { const int t = a % b; a = b; b = t; } return a; }
 
-/* the visit step of ipdm_fbp_sart: the integer in [1, S) coprime to S closest to 0.382 S, smaller on a tie; 1 when S <= 2 */
+/* the visit step of ipdm_fbp_sart_tv: the integer in [1, S) coprime to S closest to 0.382 S, smaller on a tie; 1 when S <= 2 */
 int sart_visit_step(int S)
 {
     if (S <= 2) return 1;

@@ -79,8 +79,8 @@ def visit_step(subsets):
 
 def sart(sino, flip=True, iterations=5, subsets=20, relaxation=1.0, history=False):
     """[B,2000,912] or [2000,912] line integrals (taken as f32, as the device takes them) -> [B,512,512] f64 image after
-    `iterations` sweeps of ordered-subset SART (ipdm_fbp_sart); with history=True also [B,iterations,512,512], the iterate after
-    every sweep."""
+    `iterations` sweeps of ordered-subset SART (ipdm_fbp_sart_tv with ntv = 0); with history=True also [B,iterations,512,512],
+    the iterate after every sweep."""
     sino = np.ascontiguousarray(sino, dtype=np.float32)
     if sino.ndim == 2:
         sino = sino[None]

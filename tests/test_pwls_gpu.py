@@ -1,6 +1,6 @@
 """GPU: the PWLS penalty (ipdm_fbp_pwls_penalty) and PWLS / OS-SQS (ipdm_fbp_pwls) against their fp64 C restatement
-(oracle/pwls_oracle.c), bit-for-bit frame mirroring, determinism and batch invariance, the objective's descent with one subset and
-the low-dose claim with the device operators, and convertor="PWLS" in the progressive pipeline (eager, CUDA graph,
+(oracle/pwls_oracle.c), bit-for-bit frame mirroring, determinism and batch invariance, one plan shared by every convertor at
+changing batches, the objective's descent with one subset and the low-dose claim with the device operators, and convertor="PWLS" in the progressive pipeline (eager, CUDA graph,
 simulate_low_dose)."""
 import numpy as np
 import pytest
@@ -56,8 +56,9 @@ def test_penalty_matches_the_oracle_and_mirrors(plan, cuda):
         print(f"penalty vs fp64 oracle (flip={int(flip)}): grad rel-L2 {eg:.2e}, curvature rel-L2 {ec:.2e}")
         assert eg <= PENALTY_TOL and ec <= PENALTY_TOL, (eg, ec)
     assert np.array_equal(got[True][0], got[False][0][:, ::-1]) and np.array_equal(got[True][1], got[False][1][:, ::-1])
-    with pytest.raises(ValueError):
-        plan.pwls_penalty(_dev(x, cuda)[None].contiguous(), 0.0)
+    for bad in (0.0, "0.1"):
+        with pytest.raises(ValueError):
+            plan.pwls_penalty(_dev(x, cuda)[None].contiguous(), bad)
 
 
 @pytest.mark.parametrize("init", ["zero", "fbp"])
@@ -114,6 +115,25 @@ def test_pwls_mirrors_and_is_deterministic_and_batch_invariant(plan, phantom, cu
     for bad in (dict(dose=0.0), dict(beta=-1.0), dict(delta=float("nan")), dict(init="x"), dict(subsets=7)):
         with pytest.raises(ValueError):
             plan.pwls(sb[:1].contiguous(), **dict(kw, **bad))
+
+
+def test_one_plan_serves_every_convertor_at_growing_and_shrinking_batches(phantom, cuda):
+    """A plan's per-call scratch is laid out for each call's batch and kept across convertors: calls interleaved on one plan, at
+    batches that grow and shrink, give bit for bit what the same call gives on a fresh plan."""
+    from ipdm_pytorch_b200 import engine
+    b = _dev(phantom[2][0.25], cuda)
+    sb = torch.stack([b * (1 + 0.05 * k) for k in range(16)])
+    x = torch.rand(1, 512, 512, device=cuda, generator=torch.Generator(device=cuda).manual_seed(5))
+    sart_tv = dict(ntv=20, tv_alpha=0.2, init="fbp")                # the recommended SART-TV setting
+    calls = [lambda p: p.sart(sb, **sart_tv),
+             lambda p: p.pwls(sb[:4], init="fbp", **engine.PWLS_DEFAULTS),
+             lambda p: p.tv_descent(x.clone(), 5, 1.0),
+             lambda p: p.sart(sb[:2]),
+             lambda p: p.sart(sb[:3], **sart_tv),
+             lambda p: p.pwls(sb, **engine.PWLS_DEFAULTS)]
+    shared = engine.FBPPlan()
+    for k, call in enumerate(calls):
+        assert torch.equal(call(shared), call(engine.FBPPlan())), k
 
 
 @pytest.mark.parametrize("beta", [0.0, 3e4])

@@ -87,7 +87,8 @@ def test_sart_options_parse():
 
 
 @pytest.mark.parametrize("bad", [dict(iterations=0), dict(iterations=1.5), dict(subsets=7), dict(subsets=0), dict(subsets=4000),
-                                 dict(relaxation=0.0), dict(relaxation=2.0), dict(relaxation=float("nan"))])
+                                 dict(relaxation=0.0), dict(relaxation=2.0), dict(relaxation=float("nan")), dict(relaxation=True),
+                                 dict(relaxation="0.5")])
 def test_sart_argument_checks(bad):
     from ipdm_pytorch_b200 import engine
     args = dict(engine.SART_DEFAULTS, **bad)

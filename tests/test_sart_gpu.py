@@ -1,6 +1,6 @@
 """GPU: the adjoint projector (ipdm_fbp_project_adjoint) against its fp64 C restatement and bit for bit against the forward
-projector's weights, ordered-subset SART (ipdm_fbp_sart) against its fp64 restatement, and convertor="SART" in the progressive
-pipeline (eager, CUDA graph, simulate_low_dose evaluation loop)."""
+projector's weights, ordered-subset SART (ipdm_fbp_sart_tv with ntv = 0) against its fp64 restatement, and convertor="SART" in
+the progressive pipeline (eager, CUDA graph, simulate_low_dose evaluation loop)."""
 import json
 import os
 

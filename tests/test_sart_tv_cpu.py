@@ -119,5 +119,8 @@ def test_sart_tv_argument_checks(bad):
     with pytest.raises(ValueError):
         engine.FBPPlan.check_tv_args(**args)
     with pytest.raises(ValueError):
+        engine.FBPPlan.check_sart_args(**args)
+    with pytest.raises(ValueError):
         engine.FBPPlan.check_sart_args(**engine.SART_DEFAULTS, **args)
     assert engine.FBPPlan.check_tv_args(**engine.SART_TV_DEFAULTS) == (0, 0.2, 1e-4, "zero")
+    assert engine.FBPPlan.check_sart_args(**engine.SART_TV_DEFAULTS) == (5, 100, 1.0, 0, 0.2, 1e-4, "zero")

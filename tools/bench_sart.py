@@ -1,7 +1,7 @@
 """Timing of the iterative convertor: python tools/bench_sart.py [batch ...]  (default 16 64).
 
-CUDA events around ipdm_fbp_project_adjoint, ipdm_fbp_sart (default options), one TV step (ipdm_fbp_tv_descent), SART-TV at
-the recommended setting (ipdm_fbp_sart_tv, ntv = 20, tv_alpha = 0.2, FBP start), PWLS at its defaults (ipdm_fbp_pwls, the sweeps
+CUDA events around ipdm_fbp_project_adjoint, plain SART (ipdm_fbp_sart_tv at the default options, ntv = 0), one TV step
+(ipdm_fbp_tv_descent), SART-TV at the recommended setting (ipdm_fbp_sart_tv, ntv = 20, tv_alpha = 0.2, FBP start), PWLS at its defaults (ipdm_fbp_pwls, the sweeps
 and subsets of SART, dose 0.25, FBP start) and the PWLS penalty alone (ipdm_fbp_pwls_penalty) after a warm-up of the same shape,
 which also builds SART's geometry tables.  Each timed call reads and writes buffers of its own, rotated so that one round of them exceeds the
 126 MB L2: inputs come from HBM, not from the previous call's cache lines.  Weight updates are counted from the geometry: the
